@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun)
     python bench.py --impl reference ...                      (the reference's CPU path, oracle port)
+    python bench.py ... --dump-outputs DIR                    (also write the codes of the last timed step as .npy)
 
 Workload (BASELINE.json configs[1], the prep_lm_dataset_magicodec shape): per rank, 1 h of synthetic
 16 kHz mono audio as 6 x 10 min files, encoded the way encode_audio_gpu_N.sh does it — 0.1 s chunks,
@@ -28,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import numpy as np
 import torch
@@ -59,7 +61,32 @@ def parse_args():
                     help="strong: ONE list of uneven files (the N=1 hour) sharded over the ranks with corpus.shard_by_duration")
     ap.add_argument("--stream-steps", type=int, default=5000, help="steady 20 ms steps of the streaming measurement (configs[3])")
     ap.add_argument("--no-extras", action="store_true", help="skip the auxiliary keys (e2e_cli, stereo, one-shot, decode, streaming)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the codes of the last timed step to DIR/codes_fileNNNNN.npy "
+                    "(float32; the same arguments give the same inputs, so two builds can be compared file by file)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path only")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, file_ids, codes, n_files_total: int) -> None:
+    """One .npy per file of what corpus.encode_streams returned: the int64 codes as float32 (exact below 2**24).  Past
+    DUMP_BYTES over all files, each file keeps a seeded sample of its codes and their positions (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // n_files_total - 256                     # bytes per file; 256 covers two .npy headers
+    for f, c in zip(file_ids, codes):
+        a = c.cpu().numpy()
+        name = os.path.join(out_dir, f"codes_file{f:05d}")
+        if a.size * 4 > budget:
+            pos = np.sort(np.random.default_rng(f).choice(a.size, budget // 12, replace=False))
+            np.save(name + "_positions.npy", pos.astype(np.float64))
+            a = a[pos]
+        np.save(name + ".npy", a.astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------- clocks
@@ -236,7 +263,9 @@ def main():
         file_secs = [args.file_secs] * args.files
         total_audio_secs = world * args.files * args.file_secs
         imbalance = 1.0
-    dev_files = [pkg.synth_audio(int(secs * sr), seed=1234, file_id=f, device=dev) for f, secs in zip(file_ids, file_secs)]
+    # synthesised on the host: the phase is a cumsum over the whole file, and a CUDA cumsum's summation order (so its
+    # rounding) changes from run to run, which would change the audio and the codes of every run
+    dev_files = [pkg.synth_audio(int(secs * sr), seed=1234, file_id=f).to(dev) for f, secs in zip(file_ids, file_secs)]
     host_files = [torch.empty(d.numel(), dtype=torch.float32).pin_memory() for d in dev_files]
     for h, d in zip(host_files, dev_files):
         h.copy_(d)
@@ -311,6 +340,8 @@ def main():
     if rank == 0:
         sampler.start()
     dev_ms, _, launches, _ = timed(step_device, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, file_ids, last["codes"], len(durations) if strong else world * args.files)
     # the same K steps once more with an event pair around every kernel launch: per-class device time for the
     # roofline object.  Kept out of the pass above so that `value` carries no instrumentation overhead.
     prof_ms, _, _, prof = timed(step_device, args.steps, profile=True)

@@ -11,7 +11,7 @@ import pytest
 from realtime_codec_agent_b200 import audio_io as aio
 from tests import flac_writer as fw
 
-SCIPY_WAVS = os.path.join(os.path.dirname(__import__("scipy.io").io.__file__), "tests", "data")
+SCIPY_WAVS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "wav")    # SciPy's WAV test vectors
 
 
 def _write_wav(path, sr, data, tag=1, bits=16, extensible=False):

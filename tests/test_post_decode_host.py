@@ -3,7 +3,8 @@
 * the oracle restatement (oracle/post_decode_oracle.py) reproduces the golden vectors the reference's OWN
   utils/audio_utils.py and ExternalTTSDuplexAligner produced (tests/golden/make_golden_post.py);
 * the product's host utilities and OutputChunkEmitter / ExternalTTSDuplexAligner (non-native branch)
-  reproduce them too, and — in the build container — agree with the reference modules imported unmodified.
+  reproduce them too, and agree with the stored outputs of the reference modules (tests/golden/golden_host_calls.npz)
+  and, wherever the reference is installed, with those modules imported unmodified.
 """
 import os
 
@@ -13,6 +14,7 @@ import torch
 
 import realtime_codec_agent_b200 as pkg
 from oracle import post_decode_oracle as po
+from tests.golden_calls import assert_identical, assert_matches_golden
 
 SR, CHUNK, L = 16000, 1600, 320
 
@@ -118,31 +120,54 @@ def test_aligner_reads_vocab_start_from_a_config_dir(g, tmp_path):
     assert al.codec_vocab_start == 777
 
 
-@pytest.mark.skipif(not po.reference_available(), reason="/root/reference is only mounted in the build container")
-def test_live_against_the_unmodified_reference_modules(g):
-    au = po.load_reference_module("utils.audio_utils")
+def util_calls(u):
+    """Ramps, joins and RMS normalisation over seeded inputs for three fade lengths -> {name: array}."""
     rng = np.random.default_rng(5)
+    out = {}
     for L_secs in (0.02, 0.005, 0.1):
-        n, fi, fo = au.create_crossfade_ramps(SR, L_secs)
-        for u in UTIL_SETS.values():
-            n2, fi2, fo2 = u["create_crossfade_ramps"](SR, L_secs)
-            assert n == n2 and np.array_equal(fi, fi2) and np.array_equal(fo, fo2)
-            a = rng.standard_normal(CHUNK).astype(np.float32)
-            b = rng.standard_normal(CHUNK + n).astype(np.float32)
-            assert np.array_equal(au.smooth_join(a, b, n, fi, fo), u["smooth_join"](a, b, n, fi, fo))
-            for tr in (0.05, 0.2):
-                assert np.array_equal(au.normalize_audio_rms(b, target_rms=tr), u["normalize_audio_rms"](b, target_rms=tr))
-    # the chain over a real (oracle-model) tokenizer on both sides
+        n, fi, fo = u["create_crossfade_ramps"](SR, L_secs)
+        a = rng.standard_normal(CHUNK).astype(np.float32)
+        b = rng.standard_normal(CHUNK + n).astype(np.float32)
+        out.update({f"{L_secs}_n": np.int64(n), f"{L_secs}_fade_in": fi, f"{L_secs}_fade_out": np.ascontiguousarray(fo),
+                    f"{L_secs}_join": u["smooth_join"](a, b, n, fi, fo)})
+        for tr in (0.05, 0.2):
+            out[f"{L_secs}_norm_{tr}"] = u["normalize_audio_rms"](b, target_rms=tr)
+    return out
+
+
+def chain_calls(step, history, s):
+    """The output chain fed 0.1 s (5-char) pieces of ``s`` -> {name: array}."""
+    out = {f"{i}_emitted": np.array(step(s[i:i + 5])) for i in range(0, len(s), 5)}      # a copy: buffers may be reused
+    out["history"] = np.concatenate(history())
+    return out
+
+
+def oracle_model_tokenizer_and_codes():
     from oracle.magicodec_oracle import OracleGenerator
-    from oracle.reference_wrapper import load_reference_audio_tokenizer
     model = OracleGenerator(pkg.TINY_SPEC, pkg.init_random_weights(pkg.TINY_SPEC, seed=0))
-    ref_tok = load_reference_audio_tokenizer()(codec_model=model, device="cpu")
     our_tok = pkg.AudioTokenizer(codec_model=model, device="cpu")
     s = our_tok.tokenize_audio(pkg.synth_audio(16000, file_id=2).numpy())
     our_tok.reset_context()
-    utils = {k: getattr(au, k) for k in UTIL_SETS["oracle"]}
-    chain = po.OracleOutputChain(ref_tok, 0.1, 0.02, 0.05, utils=utils)
+    return model, our_tok, s
+
+
+def test_live_against_the_unmodified_reference_modules(golden_dir):
+    """The utilities and the chain over a real (oracle-model) tokenizer, against tests/golden/golden_host_calls.npz and,
+    wherever the reference is installed, against the reference's own modules bit for bit."""
+    golden = np.load(os.path.join(golden_dir, "golden_host_calls.npz"))
+    utils = {which: util_calls(u) for which, u in UTIL_SETS.items()}
+    for got in utils.values():
+        assert_matches_golden(got, golden, "post_utils", sample=False)
+    model, our_tok, s = oracle_model_tokenizer_and_codes()
     emitter = pkg.OutputChunkEmitter(our_tok, 0.1, 0.02, 0.05)
-    for i in range(0, len(s), 5):
-        assert np.array_equal(chain.step(s[i:i + 5]), emitter.emit(s[i:i + 5]))
-    assert np.array_equal(np.concatenate(chain.history), np.concatenate(emitter.audio_history_ch1))
+    ours = chain_calls(emitter.emit, lambda: emitter.audio_history_ch1, s)
+    assert_matches_golden(ours, golden, "post_chain")
+    if po.reference_available():
+        from oracle.reference_wrapper import load_reference_audio_tokenizer
+        au = po.load_reference_module("utils.audio_utils")
+        ref_utils = {k: getattr(au, k) for k in UTIL_SETS["oracle"]}
+        for got in utils.values():
+            assert_identical(got, util_calls(ref_utils))
+        chain = po.OracleOutputChain(load_reference_audio_tokenizer()(codec_model=model, device="cpu"), 0.1, 0.02, 0.05,
+                                     utils=ref_utils)
+        assert_identical(ours, chain_calls(chain.step, lambda: chain.history, s))
