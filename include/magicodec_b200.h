@@ -241,6 +241,24 @@ int mc_op_emit_chunk(mc_handle* h, const float* wav, int32_t n_have, int32_t chu
 int mc_op_embed_distance(mc_handle* h, const float* table, int32_t K, const int64_t* ids, int32_t rows, int32_t n,
                          int64_t vocab_start, const float* ref, float* dist_out, float* mean_out, mc_stream_t stream);
 
+/* ---- offline corpus decode (the way back from a directory of codes; python -m rca_b200_loader codes_to_audio).
+ * mc_render_chunks: the agent's output chain (OutputChunkEmitter; RealtimeAgent.detokenize_output_chunk,
+ * realtime_agent_v2.py:556-579: pad_or_trim -> normalize_audio_rms (skipped when target_rms <= 0) -> smooth_join) for
+ * EVERY chunk of one mono stream in one launch; the result equals mc_op_emit_chunk run chunk by chunk, bit for bit.
+ * windows DEVICE fp32 [n_chunks, ld]: row 0 = the first chunk's decoded samples, rows i >= 1 = fade preroll ++ chunk;
+ * the last row holds last_len new samples (a ragged last chunk).  fade_in DEVICE fp32 [fade] rising ramp.
+ * out DEVICE fp32 [(n_chunks-1)*chunk + last_len] = np.concatenate(audio_history_ch1) cut to the real samples.
+ * Needs 0 < fade <= chunk, 0 < last_len <= chunk, ld >= chunk + fade. */
+int mc_render_chunks(mc_handle* h, const float* windows, int64_t ld, int32_t n_chunks, int32_t chunk, int32_t fade,
+                     int32_t last_len, float target_rms, float silence_rms_threshold, const float* fade_in, float* out,
+                     mc_stream_t stream);
+/* The CLI's writer (the reference's consumers write wav files through soundfile): planar fp32 [channels, in_ld] ->
+ * interleaved [frames][channels] as MC_PCM_S16 (clamp(rint(x * 32768), -32768, 32767), NaN -> 0: the inverse of the
+ * / 32768 of _prep_audio_for_tokenization, audio_tokenizer.py:203-215) or MC_PCM_F32.  in is a DEVICE pointer; out may
+ * be DEVICE or PINNED HOST memory. */
+int mc_op_f32_to_pcm(mc_handle* h, const float* in, int64_t in_ld, int32_t channels, int64_t frames, int32_t format, void* out,
+                     mc_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -76,6 +76,8 @@ SYMBOLS = {
     "mc_op_embed_distance": (C.c_int, [_P, _P, _I32, _P, _I32, _I32, _I64, _P, _P, _P, _P]),
     "mc_op_pcm_to_f32": (C.c_int, [_P, _P, _I32, _I32, _I32, _I64, _I32, _P, _I64, _P]),
     "mc_op_resample": (C.c_int, [_P, _P, _I64, _I32, _I64, _I32, _I32, _P, _I32, _I64, _P, _I64, _I64, _P]),
+    "mc_render_chunks": (C.c_int, [_P, _P, _I64, _I32, _I32, _I32, _I32, C.c_float, C.c_float, _P, _P, _P]),
+    "mc_op_f32_to_pcm": (C.c_int, [_P, _P, _I64, _I32, _I64, _I32, _P, _P]),
     "mc_flac_info": (C.c_int, [_P, _I64, C.POINTER(_I32), C.POINTER(_I32), C.POINTER(_I32), C.POINTER(_I64)]),
     "mc_flac_decode": (C.c_int, [_P, _I64, _P, _I64, C.POINTER(_I64)]),
     "mc_op_gemm_fused": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I32, _I32, _I32, _P, _P, _I32, _P, _P, _P, _I32, _I32, _I32, _P]),

@@ -25,6 +25,7 @@ import os
 import shutil
 import struct
 import subprocess
+import zlib
 from dataclasses import dataclass
 from typing import Callable, Optional, Tuple
 
@@ -128,6 +129,52 @@ def _read_wav(path: str, alloc: Alloc) -> PcmAudio:
         if got != nbytes:
             raise UnsupportedAudio("short read")
     return PcmAudio(sr, ch, frames, fmt, big, buf[:nbytes])
+
+
+WAV_MAX_DATA_BYTES = 0xFFFFFFFF - 36          # RIFF sizes are 32-bit; RF64 is not written
+
+
+def wav_header(sample_rate: int, channels: int, fmt: int, frames: int) -> bytes:
+    """44-byte canonical RIFF/WAVE header for interleaved PCM_S16 (format tag 1) or PCM_F32 (format tag 3) data."""
+    if fmt not in (PCM_S16, PCM_F32):
+        raise ValueError("write_wav writes 16-bit PCM or 32-bit float only")
+    width = BYTES_PER_SAMPLE[fmt]
+    data = frames * channels * width
+    if data > WAV_MAX_DATA_BYTES:
+        raise ValueError(f"{data} bytes of audio exceed the 4 GiB RIFF limit")
+    return (b"RIFF" + struct.pack("<I", 36 + data) + b"WAVE"
+            + b"fmt " + struct.pack("<IHHIIHH", 16, 1 if fmt == PCM_S16 else 3, channels, sample_rate,
+                                    sample_rate * channels * width, channels * width, 8 * width)
+            + b"data" + struct.pack("<I", data))
+
+
+def write_wav(f, pcm: np.ndarray, sample_rate: int) -> int:
+    """Write interleaved audio [frames, channels] (or [frames]) of dtype int16 or float32 as a .wav file to the binary
+    file object `f`.  Returns the crc32 of the data chunk."""
+    pcm = np.ascontiguousarray(pcm)
+    if pcm.dtype not in (np.int16, np.float32):
+        raise ValueError("write_wav writes int16 or float32 samples")
+    frames, channels = (pcm.shape[0], 1) if pcm.ndim == 1 else pcm.shape
+    body = pcm.astype(pcm.dtype.newbyteorder("<"), copy=False).reshape(-1).view(np.uint8)
+    f.write(wav_header(sample_rate, channels, PCM_S16 if pcm.dtype == np.int16 else PCM_F32, frames))
+    f.write(body)
+    return zlib.crc32(body) & 0xFFFFFFFF
+
+
+def wav_info(path: str) -> Optional[Tuple[int, int, int, int]]:
+    """(sample_rate, channels, fmt, frames) of a complete .wav file, or None when it is missing, unreadable or shorter
+    than its header says."""
+    try:
+        with open(path, "rb") as f:
+            head = f.read(44)
+            f.seek(0)
+            sr, ch, fmt, frames, _, off, nbytes = _wav_header(f)
+        declared = struct.unpack("<I", head[40:44])[0] if head[36:40] == b"data" else nbytes
+        if declared != nbytes or off + nbytes > os.path.getsize(path):
+            return None
+        return sr, ch, fmt, frames
+    except (OSError, UnsupportedAudio, struct.error):
+        return None
 
 
 # ------------------------------------------------------------------------------ NIST SPHERE
@@ -500,6 +547,48 @@ class DeviceIngest:
     def to_device(self, pcm: PcmAudio, mono: bool, host_tensor=None):
         """upload + convert."""
         return self.convert(pcm, self.upload(pcm, host_tensor), mono)
+
+    def upload_codes(self, host_tensor, nbytes: int):
+        """H2D of `nbytes` of a pinned uint8 tensor (int64 codes, the offline decode) on the copy stream -> (device bytes,
+        event); codes_on_device() hands them to the current stream."""
+        torch = self.torch
+        with torch.cuda.stream(self.copy_stream):
+            raw = torch.empty(max(nbytes, 8), dtype=torch.uint8, device=self.gen.device)[:nbytes]
+            raw.copy_(host_tensor[:nbytes], non_blocking=True)
+            done = torch.cuda.Event()
+            done.record(self.copy_stream)
+        return raw, done
+
+    def codes_on_device(self, staged, channels: int, frames: int):
+        """The uploaded codes as int64 [channels, frames], ordered after the upload on the current stream."""
+        raw, done = staged
+        main = self.torch.cuda.current_stream(self.gen.device)
+        main.wait_event(done)
+        raw.record_stream(main)
+        return raw.view(self.torch.int64).view(channels, frames)
+
+    def pcm_to_host(self, wav, fmt: int):
+        """Planar fp32 [C, T] on the device -> (interleaved [T, C] int16 / float32 numpy view of pinned memory, wait):
+        mc_op_f32_to_pcm stores straight into the pinned buffer on the current stream; wait() blocks until it has, and
+        wait.release() hands the buffer back."""
+        torch = self.torch
+        C, T = wav.shape
+        width = BYTES_PER_SAMPLE[fmt]
+        raw = self.host_buffer(max(C * T * width, 8))
+        out = raw[: C * T * width].view(torch.int16 if fmt == PCM_S16 else torch.float32)
+        if T > 0:
+            self.gen.f32_to_pcm(wav, fmt, out=out)
+        ev = torch.cuda.Event()
+        ev.record(torch.cuda.current_stream(self.gen.device))
+
+        def wait():
+            ev.synchronize()
+
+        def release():
+            self.recycle(raw)
+
+        wait.release = release
+        return out.numpy().reshape(T, C), wait
 
     def codes_to_host(self, codes):
         """Device int64 code tensors -> (pinned host tensors, wait) — async D2H on the current stream.  wait() blocks until

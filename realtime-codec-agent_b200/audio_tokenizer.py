@@ -253,6 +253,58 @@ class AudioTokenizer:
                     return fast
             return self._detokenize_audio_locked(audio_codes_str, preroll_samples)
 
+    def chunked_detokenize_audio(self, audio_codes_str: str, chunk_size_secs: float):
+        """The twin of chunked_tokenize_audio: ``detokenize_audio`` over pieces of int(chunk_size_secs * framerate * C)
+        characters, outputs concatenated -> (sampling_rate, float32 [T] or [C, T]).  Each piece is decoded from the
+        trailing context_secs of codes and only its own samples are kept, which is how the agent hears its codes.
+
+        With the B200 engine, an empty ``detokenize_context``, whole frames per piece and no hanging code, the loop runs as
+        ONE batched corpus decode (corpus.decode_streams); otherwise it runs as written.  Either way the contexts are left
+        as the loop leaves them.  The batched path runs the stateless corpus kernels, the loop's calls run on the streaming
+        session's few-rows kernels (DESIGN.md §5, "Two kernel regimes"): the two agree bit for bit with
+        ``small_m_split_k = 0`` and to the decode parity bar (SNR >= 38 dB) with the default setting."""
+        C = self.num_channels
+        step = int(chunk_size_secs * self.framerate * C)
+        if step <= 0:
+            raise ValueError(f"chunk_size_secs={chunk_size_secs} is less than one code per chunk")
+        with self._lock:
+            fast = self._chunked_detokenize_batched(audio_codes_str, step) if self._native else None
+            if fast is not None:
+                return self.sampling_rate, fast
+            parts = [self.detokenize_audio(audio_codes_str[s:s + step])[0][1] for s in range(0, len(audio_codes_str), step)]
+            if not parts:
+                return self.sampling_rate, np.zeros((0,) if C == 1 else (C, 0), dtype=np.float32)
+            return self.sampling_rate, np.concatenate(parts, axis=-1)
+
+    @torch.inference_mode()
+    def _chunked_detokenize_batched(self, text: str, step: int) -> Optional[np.ndarray]:
+        """The loop of chunked_detokenize_audio as corpus.decode_streams, taken only where it provably decodes the same
+        windows and keeps the same samples; None (nothing touched) otherwise."""
+        from . import corpus
+        C, sr = self.num_channels, self.sampling_rate
+        n = len(text)
+        if self.detokenize_context or n == 0 or step % C or n % C or self.context_frames % C:
+            return None
+        cf, hop = step // C, self.codec_model.hop
+        last = n - ((n - 1) // step) * step
+        for piece in (step, last):                                   # samples the loop keeps per piece (:283)
+            if int(piece / (self.framerate * C) * sr) != piece // C * hop:
+                return None
+        if int(self.context_secs * sr / hop) != self.context_frames // C:            # decode_streams' context in frames
+            return None
+        flat = chars_to_codes(text, 1, self.codebook_size, unicode_offset=self.unicode_offset)[0]
+        codes = np.ascontiguousarray(flat.reshape(-1, C).T)                   # [C, F]
+        dev = torch.from_numpy(codes).to(self.device)
+        wav = corpus.decode_streams(self.codec_model, [dev[c] for c in range(C)], cf * hop / sr, self.context_secs)
+        out = torch.stack(wav).cpu().numpy()
+        keep = max(last, self.context_frames)
+        self.detokenize_context = text[-keep:]
+        ctx = np.ascontiguousarray(chars_to_codes(self.detokenize_context, 1, self.codebook_size,
+                                                  unicode_offset=self.unicode_offset)[0].reshape(-1, C).T)
+        self._stream_session().load_codes(ctx[:, -(self.context_frames // C):])
+        self._session_codes_ok = True
+        return out[0] if C == 1 else out
+
     def _detokenize_on_session(self, audio_codes_str: str, preroll_samples: int):
         """Steady-state twin of _detokenize_audio_locked (same bookkeeping, same results) without a torch call; returns
         None WITHOUT touching any state when the general path has to run."""

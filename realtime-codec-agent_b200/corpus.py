@@ -144,6 +144,156 @@ def encode_streams(gen, streams: Sequence[torch.Tensor], chunk_secs: float = 0.1
     return out
 
 
+# --------------------------------------------------------------------------------- decode
+@dataclass(frozen=True)
+class DecodeWindow:
+    start_frame: int    # first frame of the code context window
+    frames: int         # frames in the window
+    keep_samples: int   # decoded samples kept: the last min(new * hop + preroll, frames * hop)
+    chunk: int          # chunk index inside the stream
+
+
+def plan_decode_stream(n_frames: int, chunk_frames: int, context_frames: int, preroll_samples: int,
+                       hop: int) -> Tuple[List[DecodeWindow], Optional[Tuple[DecodeWindow, int]]]:
+    """Windows of one code stream under the bookkeeping of a detokenize_audio loop that starts from an empty context
+    (audio_tokenizer.py:105-113): chunk i is decoded from the last max(n_new, context_frames) frames ending at it, and
+    the last n_new * hop + preroll samples (at most the whole window) are kept.
+
+    Returns (irregular windows, steady) where steady = (first window, count) describes the run of full-context,
+    full-chunk windows  start_frame = (first.chunk + j + 1) * chunk_frames - first.frames, j < count."""
+    irregular: List[DecodeWindow] = []
+    n_chunks = -(-n_frames // chunk_frames) if n_frames > 0 else 0
+    full = max(chunk_frames, context_frames)
+    steady_first, steady_count = None, 0
+    for i in range(n_chunks):
+        end = min((i + 1) * chunk_frames, n_frames)
+        n_new = end - i * chunk_frames
+        start = max(0, end - max(n_new, context_frames))
+        w = DecodeWindow(start, end - start, min(n_new * hop + preroll_samples, (end - start) * hop), i)
+        if n_new == chunk_frames and w.frames == full:
+            if steady_first is None:
+                steady_first = w
+            steady_count += 1
+        else:
+            irregular.append(w)
+    return irregular, ((steady_first, steady_count) if steady_first is not None else None)
+
+
+def _chunk_frames(gen, chunk_secs: float) -> int:
+    exact = chunk_secs * gen.sample_rate / gen.hop
+    cf = int(round(exact))
+    if cf < 1 or abs(exact - cf) > 1e-6:
+        raise ValueError(f"chunk_secs={chunk_secs} is {exact} frames; the chunked decode needs a whole number >= 1")
+    return cf
+
+
+def _decode_windows(gen, code_streams: Sequence[torch.Tensor], cf: int, context_frames: int, preroll: int,
+                    batch_size: int, causal_warmup: bool, sink) -> None:
+    """Decodes every planned window of every stream; sink(stream, first_chunk, wav [n, keep]) receives the kept samples
+    of n consecutive chunks."""
+    hop = gen.hop
+    causal_warmup = causal_warmup and int(getattr(getattr(gen, "spec", None), "window_right", 0)) == 0
+    plans = [plan_decode_stream(int(s.numel()), cf, context_frames, preroll, hop) for s in code_streams]
+
+    # steady state: the overlapping windows of a stream as an unfolded view, materialised per launch by gen.decode
+    for si, (s, (_, steady)) in enumerate(zip(code_streams, plans)):
+        if steady is None:
+            continue
+        first, count = steady
+        base = first.start_frame
+        view = s[base: base + (count - 1) * cf + first.frames].unfold(0, first.frames, cf)        # [count, frames]
+        for b0 in range(0, count, batch_size):
+            nb = min(batch_size, count - b0)
+            sink(si, first.chunk + b0, gen.decode(view[b0:b0 + nb], keep_last_samples=first.keep_samples))
+
+    # warm-up windows (start_frame 0) as prefixes of the longest one: the decoder is causal end to end (causal windowed
+    # attention, causal transposed convolutions, window-relative RoPE), so sample t of a prefix's output equals sample t
+    # of the longer window's; one full decode per stream replaces up to context/chunk launches of growing length
+    done: List[set] = [set() for _ in code_streams]
+    if causal_warmup:
+        prefix_groups: Dict[int, List[Tuple[int, List[DecodeWindow]]]] = {}
+        for si, (irr, _) in enumerate(plans):
+            warm = [w for w in irr if w.start_frame == 0]
+            if len(warm) >= 2:
+                prefix_groups.setdefault(max(w.frames for w in warm), []).append((si, warm))
+        for frames, items in prefix_groups.items():
+            for b0 in range(0, len(items), batch_size):
+                part = items[b0:b0 + batch_size]
+                wav = gen.decode(torch.stack([code_streams[si][:frames] for si, _ in part]), keep_last_samples=0)
+                for row, (si, warm) in enumerate(part):
+                    for w in warm:
+                        end = w.frames * hop
+                        sink(si, w.chunk, wav[row:row + 1, end - w.keep_samples:end])
+                        done[si].add(w.chunk)
+
+    # remaining warm-up / ragged windows: grouped across streams by (frames, keep)
+    groups: Dict[Tuple[int, int], List[Tuple[int, DecodeWindow]]] = {}
+    for si, (irr, _) in enumerate(plans):
+        for w in irr:
+            if w.chunk not in done[si]:
+                groups.setdefault((w.frames, w.keep_samples), []).append((si, w))
+    for (frames, keep), items in groups.items():
+        for b0 in range(0, len(items), batch_size):
+            part = items[b0:b0 + batch_size]
+            wav = gen.decode(torch.stack([code_streams[si][w.start_frame:w.start_frame + frames] for si, w in part]),
+                             keep_last_samples=keep)
+            for row, (si, w) in enumerate(part):
+                sink(si, w.chunk, wav[row:row + 1])
+
+
+def decode_streams(gen, code_streams: Sequence[torch.Tensor], chunk_secs: float = 0.1, context_secs: float = 2.0,
+                   batch_size: int = 256, fuse_batches: int = 1, causal_warmup: bool = True) -> List[torch.Tensor]:
+    """Chunked decode of code streams (1-D int64 device tensors) -> one fp32 waveform per stream: exactly what a loop
+    of AudioTokenizer.detokenize_audio over chunk_secs pieces returns when it starts from an empty context.  The twin
+    of encode_streams: steady windows `batch_size * fuse_batches` per engine call, warm-up chunks from ONE decode of
+    the longest warm-up prefix (causal specs only, ``window_right == 0``; any look-ahead takes the per-window path),
+    the rest grouped across streams by shape."""
+    cf = _chunk_frames(gen, chunk_secs)
+    context_frames = int(context_secs * gen.sample_rate / gen.hop)
+    pieces: List[Dict[int, torch.Tensor]] = [dict() for _ in code_streams]
+
+    def sink(si, first, wav):
+        pieces[si][first] = wav.reshape(-1)
+
+    _decode_windows(gen, code_streams, cf, context_frames, 0, batch_size * max(1, int(fuse_batches)), causal_warmup, sink)
+    return [torch.cat([p[k] for k in sorted(p)]) if p else torch.empty(0, dtype=torch.float32, device=gen.device)
+            for p in pieces]
+
+
+def render_streams(gen, code_streams: Sequence[torch.Tensor], chunk_secs: float = 0.1, context_secs: float = 2.0,
+                   fade_secs: float = 0.02, target_rms: float = 0.0, silence_rms_threshold: float = 0.003,
+                   batch_size: int = 256, fuse_batches: int = 1, causal_warmup: bool = True) -> List[torch.Tensor]:
+    """The agent's recording of each code stream: every chunk after the first decoded with preroll_samples = L, then
+    pad_or_trim -> normalize_audio_rms (target_rms > 0) -> smooth_join, i.e. np.concatenate(audio_history_ch1) of an
+    OutputChunkEmitter fed the chunk strings in order (the emitted stream shifted left by L), frames * hop samples long.
+    Windows are decoded as in decode_streams, gathered into one [n_chunks, chunk + L] matrix per stream, and the whole
+    crossfade chain is one render_chunks launch per stream."""
+    from .audio_utils import create_crossfade_ramps
+    cf = _chunk_frames(gen, chunk_secs)
+    chunk = cf * gen.hop
+    context_frames = int(context_secs * gen.sample_rate / gen.hop)
+    L, fade_in, _ = create_crossfade_ramps(gen.sample_rate, fade_secs)
+    if not 0 < L <= chunk:
+        raise ValueError(f"fade_secs={fade_secs} gives {L} fade samples; the render needs 0 < fade <= chunk ({chunk})")
+    mats = [torch.zeros((-(-int(s.numel()) // cf), chunk + L), dtype=torch.float32, device=gen.device) for s in code_streams]
+
+    def sink(si, first, wav):
+        mats[si][first:first + wav.shape[0], :wav.shape[1]] = wav
+
+    _decode_windows(gen, code_streams, cf, context_frames, L, batch_size * max(1, int(fuse_batches)), causal_warmup, sink)
+    ramp = torch.from_numpy(fade_in).to(gen.device)
+    out = []
+    for s, m in zip(code_streams, mats):
+        n = int(s.numel())
+        if n == 0:
+            out.append(torch.empty(0, dtype=torch.float32, device=gen.device))
+            continue
+        last_len = (n - (m.shape[0] - 1) * cf) * gen.hop
+        out.append(gen.render_chunks(m, chunk, ramp, last_len=last_len, target_rms=target_rms,
+                                     silence_rms_threshold=silence_rms_threshold))
+    return out
+
+
 # ------------------------------------------------------------------------------- sharding
 def shard_by_duration(durations: Sequence[float], world_size: int) -> List[List[int]]:
     """Longest-processing-time-first partition; deterministic (ties by index)."""

@@ -933,6 +933,36 @@ int mc_op_emit_chunk(mc_handle* h, const float* wav, int32_t n_have, int32_t chu
   return MC_OK;
 }
 
+int mc_render_chunks(mc_handle* h, const float* windows, int64_t ld, int32_t n_chunks, int32_t chunk, int32_t fade,
+                     int32_t last_len, float target_rms, float silence_rms_threshold, const float* fade_in, float* out,
+                     mc_stream_t stream) {
+  MC_ENTER(h);
+  if (!windows || !fade_in || !out || n_chunks < 1 || chunk < 1 || fade < 1 || fade > chunk || last_len < 1 || last_len > chunk ||
+      ld < (int64_t)chunk + fade)
+    return h->fail(MC_ERR_ARG, "mc_render_chunks: need 0 < fade (%d) <= chunk (%d), 0 < last_len (%d) <= chunk, ld (%lld) >= chunk + fade",
+                   fade, chunk, last_len, (long long)ld);
+  const double out_n = (double)(n_chunks - 1) * chunk + last_len;
+  McProfScope prof(h, 3, 0.0, out_n * 4.0 * 2.0 + (double)n_chunks * fade * 4.0, (cudaStream_t)stream);
+  mc_launch(h, emit_chunks_kernel, dim3(n_chunks), dim3(POST_THREADS), 0, (cudaStream_t)stream, windows, (long long)ld, (int)n_chunks,
+            (int)chunk, (int)fade, (int)last_len, target_rms, silence_rms_threshold, fade_in, out);
+  MC_LAUNCH_CHECK(h, "emit_chunks_kernel");
+  return MC_OK;
+}
+
+int mc_op_f32_to_pcm(mc_handle* h, const float* in, int64_t in_ld, int32_t channels, int64_t frames, int32_t format, void* out,
+                     mc_stream_t stream) {
+  MC_ENTER(h);
+  if (!in || !out || channels < 1 || frames < 1 || in_ld < frames || (format != PCM_S16 && format != PCM_F32))
+    return h->fail(MC_ERR_ARG, "mc_op_f32_to_pcm: bad arguments (format %d, channels %d, frames %lld)", format, channels, (long long)frames);
+  if (reinterpret_cast<uintptr_t>(out) & (format == PCM_S16 ? 1 : 3))
+    return h->fail(MC_ERR_ARG, "mc_op_f32_to_pcm: output is not naturally aligned");
+  McProfScope prof(h, 3, 0.0, (double)frames * channels * (4.0 + (format == PCM_S16 ? 2.0 : 4.0)), (cudaStream_t)stream);
+  f32_to_pcm_kernel<<<ew_grid(h, frames * channels, 256), 256, 0, (cudaStream_t)stream>>>(in, (long long)in_ld, channels,
+                                                                                          (long long)frames, format, out);
+  MC_LAUNCH_CHECK(h, "f32_to_pcm_kernel");
+  return MC_OK;
+}
+
 int mc_op_pcm_to_f32(mc_handle* h, const void* pcm, int32_t format, int32_t big_endian, int32_t channels, int64_t frames,
                      int32_t mix_mono, float* out, int64_t out_ld, mc_stream_t stream) {
   MC_ENTER(h);

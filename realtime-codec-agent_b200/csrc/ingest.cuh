@@ -11,6 +11,7 @@
 //   resample_poly_kernel   rational polyphase FIR: out[i] = sum_j h[(t % up) + j*up] * x[t / up - j], t = (i + pre)*down
 //                          — scipy.signal.resample_poly's upfirdn with the same (pre-padded, up-scaled) taps, fp32
 //                          accumulation in a fixed order (bit-reproducible)
+//   f32_to_pcm_kernel      the way back for the offline decode: planar fp32 -> interleaved s16 / f32 PCM
 #pragma once
 #include "engine_common.cuh"
 
@@ -81,6 +82,27 @@ pcm_to_f32_kernel(const unsigned char* __restrict__ src, int fmt, int big_endian
       out[t] = acc / static_cast<float>(C);
     } else {
       for (int c = 0; c < C; ++c) out[c * out_ld + t] = pcm_sample(src, fmt, t * C + c, big_endian);
+    }
+  }
+}
+
+// The mirror of pcm_to_f32_kernel for the offline decode's writer: planar fp32 [C, in_ld] -> interleaved [frames][C] as
+// PCM_S16 (clamp(rint(x * 32768), -32768, 32767), NaN -> 0: the exact inverse of the reference's / 32768 on int16
+// input) or PCM_F32.  `out` may be PINNED HOST memory: the stores are the device-to-host copy, at half the bytes of fp32
+// for 16-bit output, interleaved in the same pass.
+__global__ void __launch_bounds__(256)
+f32_to_pcm_kernel(const float* __restrict__ in, long long in_ld, int C, long long frames, int fmt, void* __restrict__ out) {
+  const long long total = frames * C;
+  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
+  for (long long e = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; e < total; e += stride) {
+    const long long t = e / C;
+    const int c = static_cast<int>(e - t * C);
+    const float x = in[c * in_ld + t];
+    if (fmt == PCM_S16) {
+      const float v = rintf(x * 32768.0f);
+      reinterpret_cast<short*>(out)[e] = v != v ? 0 : static_cast<short>(fminf(fmaxf(v, -32768.0f), 32767.0f));
+    } else {
+      reinterpret_cast<float*>(out)[e] = x;
     }
   }
 }

@@ -2,6 +2,7 @@
 //
 //   emit_chunk_kernel      pad_or_trim -> normalize_audio_rms -> smooth_join crossfade -> the chunk
 //                          the agent emits (realtime_agent_v2.py:556-579, utils/audio_utils.py:4-46)
+//   emit_chunks_kernel     the same chain for every chunk of a stream in one launch (offline render)
 //   embed_distance_kernel  F.embedding of code ids + distance to a reference embedding + mean
 //                          (external_tts_duplex_aligner.py:14-27)
 //
@@ -90,6 +91,57 @@ emit_chunk_kernel(const float* __restrict__ wav, int n_have, int chunk, int L, i
       fix[i] = 0.0f;
       prev_tail[i] = x(chunk - L + i);
     }
+  }
+}
+
+// The agent render of a whole stream in ONE launch (offline decode, mc_render_chunks), one CTA per chunk.  Chunk i's
+// part of the recording needs its own normalised window and the first L samples of chunk i+1's window (the crossfade
+// replaces its tail), but no earlier output: the prev_tail emit_chunk_kernel carries is always the last L samples of
+// the predecessor's own window.  Scales use the same fixed-order block_sum_f64 and the mixes the same separate
+// roundings as emit_chunk_kernel, so the result equals running that kernel chunk by chunk, bit for bit.
+//   windows [n_chunks, ld]: row 0 = the first chunk (no preroll), rows i >= 1 = L preroll ++ chunk; the last row holds
+//                           last_len new samples, the rest of it reads as zeros (pad_or_trim)
+//   out     [(n_chunks - 1) * chunk + last_len]: np.concatenate(audio_history_ch1), aligned with the codes
+__device__ __forceinline__ float render_row_scale(const float* __restrict__ w, int n, int want, float target_rms,
+                                                  float silence_thr, double* scratch) {
+  float scale = 1.0f;
+  if (target_rms > 0.0f) {
+    double ss = 0.0;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+      const double v = static_cast<double>(w[i]);
+      ss += v * v;
+    }
+    ss = block_sum_f64(ss, scratch);
+    const float rms = sqrtf(static_cast<float>(ss / static_cast<double>(want)));
+    if (rms >= silence_thr) scale = target_rms / rms;
+  }
+  return scale;
+}
+
+__global__ void __launch_bounds__(POST_THREADS)
+emit_chunks_kernel(const float* __restrict__ windows, long long ld, int n_chunks, int chunk, int L, int last_len,
+                   float target_rms, float silence_thr, const float* __restrict__ fade_in, float* __restrict__ out) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ double scratch[POST_THREADS / 32 + 1];
+  const int c = blockIdx.x;
+  const bool last = c == n_chunks - 1;
+  const int off = c ? L : 0;                                   // preroll samples in front of the chunk
+  const int len = last ? last_len : chunk;
+  const int n0 = off + len;                                    // valid samples of this row
+  const float* w0 = windows + static_cast<long long>(c) * ld;
+  const float s0 = render_row_scale(w0, n0, c ? chunk + L : chunk, target_rms, silence_thr, scratch);
+  const float* w1 = last ? w0 : w0 + ld;
+  const float s1 = last ? 1.0f
+                        : render_row_scale(w1, L + (c + 1 == n_chunks - 1 ? last_len : chunk), chunk + L, target_rms,
+                                           silence_thr, scratch);
+  float* o = out + static_cast<long long>(c) * chunk;
+  for (int k = threadIdx.x; k < len; k += blockDim.x) {
+    float e = __fmul_rn(w0[off + k], s0);
+    const int j = k - (chunk - L);
+    // separate roundings like numpy's tail1 * fade_out + head2 * fade_in (no FMA contraction)
+    if (!last && j >= 0) e = __fadd_rn(__fmul_rn(e, fade_in[L - 1 - j]), __fmul_rn(__fmul_rn(w1[j], s1), fade_in[j]));
+    o[k] = e;
   }
 }
 

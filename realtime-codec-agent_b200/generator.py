@@ -458,6 +458,46 @@ class B200Generator:
             nat.check(self._lib, self._handle, rc, "mc_decode")
         return wav
 
+    def render_chunks(self, windows: torch.Tensor, chunk: int, fade_in: torch.Tensor, last_len: Optional[int] = None,
+                      target_rms: float = 0.0, silence_rms_threshold: float = 0.003) -> torch.Tensor:
+        """The agent's output chain over every chunk of one mono stream in ONE launch (mc_render_chunks).
+        windows fp32 [n_chunks, ld >= chunk + L] on the device: row 0 = the first chunk, rows i >= 1 = L preroll ++ chunk;
+        fade_in fp32 [L] (create_crossfade_ramps).  Returns fp32 [(n_chunks-1)*chunk + last_len] =
+        np.concatenate(OutputChunkEmitter.audio_history_ch1) cut to the real samples of the last chunk."""
+        windows = windows.to(self.device, F32).contiguous()
+        n_chunks, ld = windows.shape
+        last_len = chunk if last_len is None else int(last_len)
+        fade_in = fade_in.to(self.device, F32).contiguous()
+        out = torch.empty(((n_chunks - 1) * chunk + last_len,), dtype=F32, device=self.device)
+        with self._serial():
+            rc = self._lib.mc_render_chunks(self._handle, windows.data_ptr(), ld, n_chunks, chunk, fade_in.numel(),
+                                            last_len, float(target_rms), float(silence_rms_threshold), fade_in.data_ptr(),
+                                            out.data_ptr(), self._stream())
+            nat.check(self._lib, self._handle, rc, "mc_render_chunks")
+        return out
+
+    PCM_S16, PCM_F32 = 1, 4                     # MC_PCM_* of include/magicodec_b200.h
+
+    def f32_to_pcm(self, wav: torch.Tensor, fmt: int = 1, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Planar fp32 [C, T] (or [T]) on the device -> interleaved PCM [T, C] (mc_op_f32_to_pcm): int16 for
+        fmt = PCM_S16 (clamp(rint(x * 32768)), NaN -> 0), float32 for PCM_F32.  `out` may be a pinned host tensor of
+        that dtype with at least T*C elements; the kernel writes into it directly (wait on the stream before reading)."""
+        if wav.dim() == 1:
+            wav = wav[None]
+        if wav.stride(-1) != 1:
+            wav = wav.contiguous()
+        C, T = wav.shape
+        dtype = torch.int16 if fmt == self.PCM_S16 else F32
+        if out is None:
+            out = torch.empty((T, C), dtype=dtype, device=self.device)
+        if out.dtype != dtype or out.numel() < T * C or not out.is_contiguous():
+            raise ValueError(f"f32_to_pcm: out must be a contiguous {dtype} buffer of at least {T * C} elements")
+        with self._serial():
+            rc = self._lib.mc_op_f32_to_pcm(self._handle, wav.data_ptr(), wav.stride(0) if C > 1 else T, C, T, int(fmt),
+                                            out.data_ptr(), self._stream())
+            nat.check(self._lib, self._handle, rc, "mc_op_f32_to_pcm")
+        return out.view(-1)[: T * C].view(T, C)
+
     def vq_search(self, z: torch.Tensor, return_margin: bool = False):
         z = z.to(self.device, F32).contiguous()
         M = z.shape[0]
