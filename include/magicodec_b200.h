@@ -188,6 +188,16 @@ int mc_stream_set_emit(mc_stream* s, int32_t chunk_samples, int32_t fade_samples
                        float silence_rms_threshold, const float* fade_in);
 int mc_stream_push_codes_emit(mc_stream* s, const int64_t* codes, int32_t n, float* out, int32_t* had_prev,
                               mc_stream_t stream);
+/* The same chain for the mono sessions of a pool, n of them in one launch (one CUDA graph: decoder + emit_chunk_pool_kernel).
+ * set_emit: the parameters of mc_stream_set_emit, shared by every slot; every slot forgets its previous chunk.
+ * push_codes_emit: codes HOST int64 [n][len] with len * hop == chunk; out HOST fp32 [n][2*chunk + L], item j laid out as
+ * mc_stream_push_codes_emit's block.  Per slot the semantics are those of mc_stream_push_codes_emit; all slots of one
+ * call must share the context length and *had_prev (first chunks and continuing chunks go in separate calls).
+ * mc_pool_reset(slot, codes != 0) also forgets that slot's previous chunk. */
+int mc_pool_set_emit(mc_pool* p, int32_t chunk_samples, int32_t fade_samples, float target_rms, float silence_rms_threshold,
+                     const float* fade_in);
+int mc_pool_push_codes_emit(mc_pool* p, const int32_t* slots, int32_t n, const int64_t* codes, int32_t len, float* out,
+                            int32_t* had_prev, mc_stream_t stream);
 
 /* ids DEVICE int64 [rows, n] (LM token ids; code = id - vocab_start, clamped to the codebook).
  * dist_out DEVICE fp32 [rows] (optional) = mean_j ||E[code_j] - ref||_2, ref DEVICE fp32 [dq] (NULL = 0);

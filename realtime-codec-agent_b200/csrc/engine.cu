@@ -1529,9 +1529,30 @@ struct mc_pool {
   bool use_graphs = true;
   cudaStream_t own = nullptr;
   cudaEvent_t order_ev = nullptr;
+  // post-decode emit chain shared by every slot (mc_pool_set_emit / mc_pool_push_codes_emit)
+  int emit_chunk = 0, emit_fade = 0;
+  float emit_target_rms = 0.f, emit_silence_thr = 0.f;
+  std::vector<int> emit_has_prev;  // per slot
+  float* emit_fade_in = nullptr;   // device [fade]
+  float* emit_prev_tails = nullptr;// device [max_sessions][fade]
+  float* pin_emit = nullptr;       // pinned [max_sessions][2*chunk + fade]
 };
 
 namespace {
+void pool_drop_graphs(mc_pool* p) {
+  for (auto& kv : p->graphs)
+    if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
+  p->graphs.clear();
+}
+
+void pool_free_emit(mc_pool* p) {
+  if (p->emit_fade_in) cudaFree(p->emit_fade_in);
+  if (p->emit_prev_tails) cudaFree(p->emit_prev_tails);
+  if (p->pin_emit) cudaFreeHost(p->pin_emit);
+  p->emit_fade_in = p->emit_prev_tails = p->pin_emit = nullptr;
+  p->emit_chunk = p->emit_fade = 0;
+}
+
 int pool_check_slots(mc_pool* p, const int32_t* slots, int n, const std::vector<int>& lens, int* common_len, const char* what) {
   mc_handle* h = p->h;
   if (!slots || n < 1 || n > p->max_sessions) return h->fail(MC_ERR_ARG, "%s: need 1..%d sessions, got %d", what, p->max_sessions, n);
@@ -1552,8 +1573,8 @@ extern "C" {
 
 int mc_pool_destroy(mc_pool* p) {
   if (!p) return MC_OK;
-  for (auto& kv : p->graphs)
-    if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
+  pool_drop_graphs(p);
+  pool_free_emit(p);
   for (int i = 0; i < 2; ++i) { if (p->audio[i]) cudaFree(p->audio[i]); if (p->codes[i]) cudaFree(p->codes[i]); }
   for (void* d : {(void*)p->dev_chunk, (void*)p->batch_audio, (void*)p->dev_codes_in, (void*)p->batch_codes, (void*)p->dev_table,
                   (void*)p->dev_codes_out, (void*)p->dev_wav_out})
@@ -1581,6 +1602,7 @@ int mc_pool_create(mc_handle* h, int32_t channels, int32_t context_samples, int3
   if (p->cap_frames > h->spec.max_positions) { delete p; return h->fail(MC_ERR_ARG, "mc_pool_create: context exceeds RoPE table"); }
   p->audio_len.assign(max_sessions, 0); p->code_len.assign(max_sessions, 0);
   p->acur.assign(max_sessions, 0); p->ccur.assign(max_sessions, 0);
+  p->emit_has_prev.assign(max_sessions, 0);
   const size_t rows = (size_t)max_sessions * channels;
   const size_t ab = rows * p->cap_samples * 4, cb = rows * p->cap_frames * 8;
   cudaError_t e = cudaSuccess;
@@ -1603,7 +1625,7 @@ int mc_pool_create(mc_handle* h, int32_t channels, int32_t context_samples, int3
 int mc_pool_reset(mc_pool* p, int32_t slot, int32_t audio, int32_t codes) {
   if (!p || slot < 0 || slot >= p->max_sessions) return MC_ERR_ARG;
   if (audio) p->audio_len[slot] = 0;
-  if (codes) p->code_len[slot] = 0;
+  if (codes) { p->code_len[slot] = 0; p->emit_has_prev[slot] = 0; }
   return MC_OK;
 }
 
@@ -1617,11 +1639,7 @@ int mc_pool_context_len(mc_pool* p, int32_t slot, int32_t* audio_len, int32_t* c
 int mc_pool_set_graphs(mc_pool* p, int32_t enabled) {
   if (!p) return MC_ERR_ARG;
   p->use_graphs = enabled != 0;
-  if (!enabled) {
-    for (auto& kv : p->graphs)
-      if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
-    p->graphs.clear();
-  }
+  if (!enabled) pool_drop_graphs(p);
   return MC_OK;
 }
 
@@ -1703,6 +1721,96 @@ int mc_pool_push_codes(mc_pool* p, const int32_t* slots, int32_t n, const int64_
   memcpy(wav_out, p->pin_wav_out, (size_t)rows * keep * 4);
   if (samples_out) *samples_out = keep;
   for (int j = 0; j < n; ++j) { p->ccur[slots[j]] ^= 1; p->code_len[slots[j]] = new_len; }
+  return MC_OK;
+}
+
+/* The emit chain of mc_stream_set_emit, shared by every slot of the pool; every slot forgets its previous chunk. */
+int mc_pool_set_emit(mc_pool* p, int32_t chunk_samples, int32_t fade_samples, float target_rms, float silence_rms_threshold,
+                     const float* fade_in) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  if (chunk_samples < 1 || fade_samples < 1 || fade_samples > chunk_samples || !fade_in)
+    return h->fail(MC_ERR_ARG, "mc_pool_set_emit: need 0 < fade (%d) <= chunk (%d) and a ramp", fade_samples, chunk_samples);
+  if (chunk_samples + fade_samples > p->cap_samples)
+    return h->fail(MC_ERR_ARG, "mc_pool_set_emit: chunk + fade exceeds the session capacity %d", p->cap_samples);
+  MC_CUDA(h, cudaStreamSynchronize(p->own));
+  pool_drop_graphs(p);   // the captured kernels carry the old parameters and buffers
+  pool_free_emit(p);
+  std::fill(p->emit_has_prev.begin(), p->emit_has_prev.end(), 0);
+  const size_t fb = (size_t)fade_samples * 4;
+  cudaError_t e = cudaMalloc(&p->emit_fade_in, fb);
+  if (e == cudaSuccess) e = cudaMalloc(&p->emit_prev_tails, fb * p->max_sessions);
+  if (e == cudaSuccess) e = cudaMallocHost(&p->pin_emit, (size_t)p->max_sessions * (2 * chunk_samples + fade_samples) * 4);
+  if (e == cudaSuccess) e = cudaMemcpy(p->emit_fade_in, fade_in, fb, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemset(p->emit_prev_tails, 0, fb * p->max_sessions);
+  if (e != cudaSuccess) { pool_free_emit(p); return h->fail(MC_ERR_NOMEM, "mc_pool_set_emit: %s", cudaGetErrorString(e)); }
+  p->emit_chunk = chunk_samples; p->emit_fade = fade_samples;
+  p->emit_target_rms = target_rms; p->emit_silence_thr = silence_rms_threshold;
+  return MC_OK;
+}
+
+/* mc_stream_push_codes_emit for n sessions in one launch.  codes: HOST int64 [n][len]; out: HOST fp32 [n][2*chunk + fade],
+ * item j in the layout of mc_stream_push_codes_emit.  Every slot of one call must be at the same point of its stream:
+ * all first chunks (empty code context) or all continuing ones. */
+int mc_pool_push_codes_emit(mc_pool* p, const int32_t* slots, int32_t n, const int64_t* codes, int32_t len, float* out,
+                            int32_t* had_prev, mc_stream_t stream_) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  int old_len = 0;
+  MC_TRY(pool_check_slots(p, slots, n, p->code_len, &old_len, "mc_pool_push_codes_emit"));
+  if (!codes || !out || len < 1) return h->fail(MC_ERR_ARG, "mc_pool_push_codes_emit: bad arguments");
+  if (len > p->cap_frames) return h->fail(MC_ERR_ARG, "mc_pool_push_codes_emit: %d frames exceed the capacity %d", len, p->cap_frames);
+  if (p->C != 1) return h->fail(MC_ERR_ARG, "mc_pool_push_codes_emit: the emit chain is mono (pad_or_trim rejects [C,T])");
+  if (p->emit_chunk <= 0) return h->fail(MC_ERR_STATE, "mc_pool_push_codes_emit: call mc_pool_set_emit first");
+  int hop = 1;
+  for (int i = 0; i < h->spec.n_convs; ++i) hop *= h->spec.conv_strides[i];
+  const int chunk = p->emit_chunk, fade = p->emit_fade, cap = p->cap_frames;
+  if (len * hop != chunk)
+    return h->fail(MC_ERR_ARG, "mc_pool_push_codes_emit: %d codes decode to %d samples, chunk is %d", len, len * hop, chunk);
+  const int new_len = std::min(old_len + len, std::max(len, p->ctx_frames));
+  const int keep_old = new_len - len;
+  const int keep = std::min(new_len * hop, chunk + fade);
+  // the stream's rules (realtime_agent_v2.py:566-568) for every slot, before any work or state change
+  for (int j = 0; j < n; ++j) {
+    if (p->emit_has_prev[slots[j]] && keep != chunk + fade)
+      return h->fail(MC_ERR_STATE, "mc_pool_push_codes_emit: slot %d: only %d decoded samples for chunk %d + fade %d", slots[j], keep,
+                     chunk, fade);
+    if (!p->emit_has_prev[slots[j]] && keep != chunk)
+      return h->fail(MC_ERR_STATE, "mc_pool_push_codes_emit: slot %d: the first emitted chunk needs an empty code context (reset first)",
+                     slots[j]);
+  }
+  const int has_prev = p->emit_has_prev[slots[0]];
+  for (int j = 1; j < n; ++j)
+    if (p->emit_has_prev[slots[j]] != has_prev)
+      return h->fail(MC_ERR_ARG, "mc_pool_push_codes_emit: slots %d and %d mix a first chunk with a continuing one; batch them separately",
+                     slots[0], slots[j]);
+  MC_CUDA(h, cudaEventRecord(p->order_ev, (cudaStream_t)stream_));
+  MC_CUDA(h, cudaStreamWaitEvent(p->own, p->order_ev, 0));
+  cudaStream_t stream = p->own;
+  const int block = 2 * chunk + fade;
+  for (int j = 0; j < n; ++j) memcpy(p->pin_codes_in + (size_t)j * cap, codes + (size_t)j * len, (size_t)len * 8);
+  for (int j = 0; j < n; ++j) { p->pin_table[2 * j] = slots[j]; p->pin_table[2 * j + 1] = p->ccur[slots[j]]; }
+  auto body = [&]() -> int {
+    MC_CUDA(h, cudaMemcpyAsync(p->dev_table, p->pin_table, (size_t)n * 8, cudaMemcpyHostToDevice, stream));
+    MC_CUDA(h, cudaMemcpy2DAsync(p->dev_codes_in, (size_t)cap * 8, p->pin_codes_in, (size_t)cap * 8, (size_t)len * 8, n, cudaMemcpyHostToDevice, stream));
+    pool_roll_kernel<long long><<<dim3((new_len + 255) / 256, n), 256, 0, stream>>>(
+        p->dev_table, 1, cap, old_len, keep_old, len, reinterpret_cast<long long*>(p->codes[0]), reinterpret_cast<long long*>(p->codes[1]),
+        reinterpret_cast<const long long*>(p->dev_codes_in), reinterpret_cast<long long*>(p->batch_codes), new_len);
+    MC_LAUNCH_CHECK(h, "pool_roll_kernel");
+    MC_TRY(decode_impl(h, p->batch_codes, nullptr, n, new_len, keep, p->dev_wav_out, stream));
+    mc_launch(h, emit_chunk_pool_kernel, dim3(n), dim3(POST_THREADS), 0, stream, (const float*)p->dev_wav_out, (long long)keep, keep,
+              (const int*)p->dev_table, chunk, fade, has_prev, p->emit_target_rms, p->emit_silence_thr, (const float*)p->emit_fade_in,
+              p->emit_prev_tails, p->pin_emit);                  // the blocks land in pinned host memory directly
+    MC_LAUNCH_CHECK(h, "emit_chunk_pool_kernel");
+    return MC_OK;
+  };
+  MC_TRY(run_or_replay(p, std::make_tuple(2 + has_prev, old_len, len, keep, n), stream, body));
+  MC_CUDA(h, cudaStreamSynchronize(stream));
+  memcpy(out, p->pin_emit, (size_t)n * block * 4);
+  if (had_prev) *had_prev = has_prev;
+  for (int j = 0; j < n; ++j) { p->ccur[slots[j]] ^= 1; p->code_len[slots[j]] = new_len; p->emit_has_prev[slots[j]] = 1; }
   return MC_OK;
 }
 

@@ -2,6 +2,7 @@
 //
 //   emit_chunk_kernel      pad_or_trim -> normalize_audio_rms -> smooth_join crossfade -> the chunk
 //                          the agent emits (realtime_agent_v2.py:556-579, utils/audio_utils.py:4-46)
+//   emit_chunk_pool_kernel the same chain for every session of a session-pool batch in one launch
 //   emit_chunks_kernel     the same chain for every chunk of a stream in one launch (offline render)
 //   embed_distance_kernel  F.embedding of code ids + distance to a reference embedding + mean
 //                          (external_tts_duplex_aligner.py:14-27)
@@ -43,13 +44,9 @@ __device__ __forceinline__ double block_sum_f64(double v, double* scratch /*[POS
 //       [chunk + L, 2*chunk + L)  the new history chunk
 // has_prev = 0 (first chunk of a session): n_have = chunk (no preroll was available); the chunk is
 // emitted delayed by L behind L zeros and becomes the history as is.
-__global__ void __launch_bounds__(POST_THREADS)
-emit_chunk_kernel(const float* __restrict__ wav, int n_have, int chunk, int L, int has_prev, float target_rms,
-                  float silence_thr, const float* __restrict__ fade_in, float* __restrict__ prev_tail,
-                  float* __restrict__ out) {
-  pdl_launch_dependents();
-  pdl_wait();
-  __shared__ double scratch[POST_THREADS / 32 + 1];
+__device__ __forceinline__ void emit_chunk_body(const float* __restrict__ wav, int n_have, int chunk, int L, int has_prev,
+                                                float target_rms, float silence_thr, const float* __restrict__ fade_in,
+                                                float* __restrict__ prev_tail, float* __restrict__ out, double* scratch) {
   const int want = has_prev ? chunk + L : chunk;       // pad_or_trim target (right pad with zeros / trim)
   const int n = min(n_have, want);
   float scale = 1.0f;
@@ -92,6 +89,35 @@ emit_chunk_kernel(const float* __restrict__ wav, int n_have, int chunk, int L, i
       prev_tail[i] = x(chunk - L + i);
     }
   }
+}
+
+__global__ void __launch_bounds__(POST_THREADS)
+emit_chunk_kernel(const float* __restrict__ wav, int n_have, int chunk, int L, int has_prev, float target_rms,
+                  float silence_thr, const float* __restrict__ fade_in, float* __restrict__ prev_tail,
+                  float* __restrict__ out) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ double scratch[POST_THREADS / 32 + 1];
+  emit_chunk_body(wav, n_have, chunk, L, has_prev, target_rms, silence_thr, fade_in, prev_tail, out, scratch);
+}
+
+// The same chain for the n sessions of one session-pool batch (mc_pool_push_codes_emit), one CTA per batch item j:
+//   wav       [n, ld]                    decoded windows, n_have samples each
+//   table     [n][2]                     table[2j] = pool slot of item j (the table pool_roll_kernel reads)
+//   prev_tails[max_sessions, L]          per-slot crossfade tails, updated in place
+//   out       [n, 2*chunk + L]           item j's block in emit_chunk_kernel's layout
+// has_prev is shared by the whole batch (the engine groups first chunks apart from continuing ones).
+__global__ void __launch_bounds__(POST_THREADS)
+emit_chunk_pool_kernel(const float* __restrict__ wav, long long ld, int n_have, const int* __restrict__ table, int chunk,
+                       int L, int has_prev, float target_rms, float silence_thr, const float* __restrict__ fade_in,
+                       float* __restrict__ prev_tails, float* __restrict__ out) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ double scratch[POST_THREADS / 32 + 1];
+  const int j = blockIdx.x;
+  const long long slot = table[2 * j];
+  emit_chunk_body(wav + j * ld, n_have, chunk, L, has_prev, target_rms, silence_thr, fade_in, prev_tails + slot * L,
+                  out + static_cast<long long>(j) * (2 * chunk + L), scratch);
 }
 
 // The agent render of a whole stream in ONE launch (offline decode, mc_render_chunks), one CTA per chunk.  Chunk i's

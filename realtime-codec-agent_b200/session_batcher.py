@@ -12,9 +12,13 @@ string context, the ``[-0:]`` / hanging-code quirks of audio_tokenizer.py:99-101
 outputs are what its own ``AudioTokenizer`` would have returned.  Sessions whose contexts differ in length (a stream
 that has just started next to one in steady state) are grouped by length: one launch per group.
 
-``ThreadedSessionBatcher`` adds the tts_server.py calling pattern: request threads call
-``tokenize_audio(session, chunk)`` and block; a dispatcher thread collects whatever arrived within ``max_wait_ms``
-and runs it as one batch.
+``SessionBatcher.emit_output_chunks`` is ``OutputChunkEmitter.emit`` for many agents at once: decoder, ``pad_or_trim``,
+``normalize_audio_rms`` and ``smooth_join`` of every session of a group run as ONE engine call (``mc_pool_push_codes_emit``,
+one CUDA graph), and each session keeps the agent's ``audio_history_ch1``.
+
+``ThreadedSessionBatcher`` adds the tts_server.py calling pattern: request threads call ``tokenize_audio_one``,
+``detokenize_audio_one`` or ``emit_output_chunk_one`` and block; a dispatcher thread collects whatever arrived within
+``max_wait_ms`` and runs it as one batch per kind.
 """
 from __future__ import annotations
 
@@ -26,6 +30,7 @@ from typing import Dict, List, Optional, Tuple
 import numpy as np
 
 from . import _native as nat
+from .audio_utils import create_crossfade_ramps
 from .codec_chars import UNICODE_OFFSET_LARGE, chars_to_codes, codes_to_chars
 
 
@@ -76,6 +81,30 @@ class SessionPool:
             nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_push_codes")
         return out[: len(slots) * self.channels * got.value].reshape(len(slots), self.channels, got.value)
 
+    def set_emit(self, chunk_samples: int, fade_samples: int, target_rms: float, silence_rms_threshold: float, fade_in) -> None:
+        """Arm the post-decode chain for every slot (mc_pool_set_emit); every slot forgets its previous chunk."""
+        ramp = np.ascontiguousarray(fade_in, dtype=np.float32)
+        if ramp.shape != (fade_samples,):
+            raise ValueError("fade_in must hold fade_samples values")
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_set_emit(self._p, chunk_samples, fade_samples, float(target_rms),
+                                                float(silence_rms_threshold), ramp.ctypes.data)
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_set_emit")
+        self._emit_floats = 2 * chunk_samples + fade_samples
+
+    def push_codes_emit(self, slots, codes: np.ndarray) -> Tuple[np.ndarray, bool]:
+        """codes int64 [n, len] -> (float32 [n, 2*chunk + fade]: per session emitted ++ cross-faded tail ++ new history
+        chunk, had_prev shared by the batch)."""
+        slots = np.ascontiguousarray(slots, dtype=np.int32)
+        codes = np.ascontiguousarray(codes, dtype=np.int64).reshape(len(slots), -1)
+        out = np.empty((len(slots), getattr(self, "_emit_floats", 0)), dtype=np.float32)
+        had = C.c_int32(0)
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_push_codes_emit(self._p, slots.ctypes.data, len(slots), codes.ctypes.data, codes.shape[1],
+                                                       out.ctypes.data, C.byref(had), self.gen._stream())
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_push_codes_emit")
+        return out, bool(had.value)
+
     def __del__(self):
         try:
             if getattr(self, "_p", None) and self.gen._handle:
@@ -90,6 +119,7 @@ class _SessionState:
         self.slot = slot
         self.audio_len = 0            # samples in the rolling audio context (len(tokenize_context[-1]))
         self.detok_context = ""       # the code-string context (detokenize_context)
+        self.history: List[np.ndarray] = []   # the agent's audio_history_ch1 (emit_output_chunks)
 
 
 class SessionBatcher:
@@ -111,6 +141,7 @@ class SessionBatcher:
         self._sessions: Dict[int, _SessionState] = {}
         self._next_id = 0
         self._lock = threading.RLock()
+        self._emit: Optional[Tuple[int, int]] = None   # (chunk samples, fade samples) once arm_emit ran
 
     # ---- session lifetime
     def open_session(self) -> int:
@@ -132,7 +163,7 @@ class SessionBatcher:
         with self._lock:
             st = self._sessions[sid]
             self.pool.reset(st.slot)
-            st.audio_len, st.detok_context = 0, ""
+            st.audio_len, st.detok_context, st.history = 0, "", []
 
     # ---- encode
     def tokenize_audio(self, chunks: Dict[int, np.ndarray]) -> Dict[int, str]:
@@ -207,26 +238,101 @@ class SessionBatcher:
                     out[sid] = ((self.sampling_rate, (w[0] if C_ == 1 else w).copy()), hanging[sid], preroll_left)
             return out
 
+    # ---- decode + the agent's output chain
+    def arm_emit(self, chunk_size_secs: float = 0.1, chunk_fade_secs: float = 0.02, target_volume_rms: float = 0.0,
+                 silence_rms_threshold: float = 0.003) -> None:
+        """OutputChunkEmitter's parameters, shared by every session (agents cloned from one RealtimeAgentConfig).
+        Every session forgets its previous chunk and its recording."""
+        if self.num_channels != 1:
+            raise ValueError("the agent's output chain is mono (pad_or_trim rejects [C,T] arrays)")
+        chunk = int(chunk_size_secs * self.sampling_rate)                                   # realtime_agent_v2.py:129
+        L, fade_in, _ = create_crossfade_ramps(self.sampling_rate, fade_secs=chunk_fade_secs)   # :131
+        if not 0 < L <= chunk:
+            raise ValueError("chunk_fade_secs must give 0 < fade samples <= chunk samples")
+        with self._lock:
+            self.pool.set_emit(chunk, L, target_volume_rms, silence_rms_threshold, fade_in)
+            self._emit = (chunk, L)
+            for st in self._sessions.values():
+                st.history = []
+
+    def audio_history_ch1(self, sid: int) -> List[np.ndarray]:
+        """The session's audio_history_ch1: ``np.concatenate`` of it is the agent's recording (realtime_agent_v2.py:744)."""
+        with self._lock:
+            return self._sessions[sid].history
+
+    def emit_output_chunks(self, strings: Dict[int, str]) -> Dict[int, np.ndarray]:
+        """{session: output code string of one chunk} -> {session: float32 [chunk]}, each exactly what that session's own
+        ``OutputChunkEmitter.emit`` returns; the code contexts advance as in ``detokenize_audio``.  Sessions are grouped by
+        code-context length, one engine call per group."""
+        with self._lock:
+            if self._emit is None:
+                raise ValueError("call arm_emit first")
+            chunk, L = self._emit
+            hop = self.gen.hop
+            new_codes, groups = {}, {}
+            for sid, s in strings.items():                       # validate everything before any state changes
+                if sid not in self._sessions:
+                    raise KeyError(f"unknown session {sid}")
+                st = self._sessions[sid]
+                if len(s) * hop != chunk:
+                    raise ValueError(f"session {sid}: {len(s)} codes decode to {len(s) * hop} samples, the chunk is {chunk}")
+                if not st.history and st.detok_context:
+                    raise ValueError(f"session {sid}: the first emitted chunk needs an empty code context (reset_context first)")
+                new_codes[sid] = chars_to_codes(s, 1, self.codebook_size, unicode_offset=self.unicode_offset)[0]
+                ctx_frames_before = self.pool.context_len(st.slot)[1]
+                groups.setdefault((ctx_frames_before, bool(st.history)), []).append(sid)
+            for sid, s in strings.items():
+                st = self._sessions[sid]
+                st.detok_context = (st.detok_context + s)[-max(len(s), self.context_frames):]
+            out = {}
+            for (_, has_prev), sids in groups.items():
+                blocks, had_prev = self.pool.push_codes_emit([self._sessions[s].slot for s in sids],
+                                                             np.stack([new_codes[s] for s in sids]))
+                if had_prev != has_prev:
+                    raise RuntimeError("emit chain state diverged from audio_history_ch1")
+                for j, sid in enumerate(sids):                   # OutputChunkEmitter._emit_native, session by session
+                    block, hist = blocks[j], self._sessions[sid].history
+                    if had_prev:
+                        hist[-1] = np.concatenate((hist[-1][:chunk - L], block[chunk:chunk + L]))
+                    hist.append(block[chunk + L:].copy())
+                    out[sid] = block[:chunk].copy()
+            return out
+
 
 class ThreadedSessionBatcher(SessionBatcher):
-    """tts_server.py's calling pattern: every request thread calls ``tokenize_audio_one(session, chunk)`` and blocks;
-    the dispatcher thread runs everything that arrived within ``max_wait_ms`` as one batch."""
+    """tts_server.py's calling pattern: every request thread calls ``tokenize_audio_one(session, chunk)``,
+    ``detokenize_audio_one(session, codes)`` or ``emit_output_chunk_one(session, codes)`` and blocks; each tick the
+    dispatcher thread runs everything that arrived within ``max_wait_ms``: the encode batch, then one decode batch per
+    ``preroll_samples`` value, then the emit batch.  A session has at most one request of each kind in a tick; later
+    ones wait for the next tick.  Encode and decode contexts are independent, so the order of the kinds changes no
+    result."""
 
     def __init__(self, *args, max_wait_ms: float = 2.0, **kw):
         super().__init__(*args, **kw)
         self.max_wait = max_wait_ms / 1e3
         self._cv = threading.Condition()
-        self._pending: List[Tuple[int, np.ndarray, Future]] = []
+        self._pending: List[Tuple[tuple, int, object, Future]] = []   # (kind, session, payload, future)
         self._stop = False
         self._thread = threading.Thread(target=self._run, daemon=True)
         self._thread.start()
 
-    def tokenize_audio_one(self, sid: int, chunk: np.ndarray, timeout: Optional[float] = 30.0) -> str:
+    def _submit(self, kind: tuple, sid: int, payload, timeout: Optional[float]):
         fut: Future = Future()
         with self._cv:
-            self._pending.append((sid, chunk, fut))
+            self._pending.append((kind, sid, payload, fut))
             self._cv.notify()
         return fut.result(timeout=timeout)
+
+    def tokenize_audio_one(self, sid: int, chunk: np.ndarray, timeout: Optional[float] = 30.0) -> str:
+        return self._submit(("encode",), sid, chunk, timeout)
+
+    def detokenize_audio_one(self, sid: int, code_str: str, preroll_samples: int = 0, timeout: Optional[float] = 30.0):
+        """-> ((sr, wav), end_hanging, preroll_left), as SessionBatcher.detokenize_audio gives it for this session."""
+        return self._submit(("decode", int(preroll_samples)), sid, code_str, timeout)
+
+    def emit_output_chunk_one(self, sid: int, code_str: str, timeout: Optional[float] = 30.0) -> np.ndarray:
+        """The session's OutputChunkEmitter.emit(code_str), batched with the other sessions' emits of the tick."""
+        return self._submit(("emit",), sid, code_str, timeout)
 
     def shutdown(self) -> None:
         with self._cv:
@@ -244,24 +350,37 @@ class ThreadedSessionBatcher(SessionBatcher):
                     return
             time.sleep(self.max_wait)                      # let the other streams' chunks of this tick arrive
             with self._cv:
-                batch, rest, seen = [], [], set()
-                for item in self._pending:                 # one chunk per session per batch, in arrival order
-                    (batch if item[0] not in seen else rest).append(item)
-                    seen.add(item[0])
+                batches: Dict[tuple, List[Tuple[int, object, Future]]] = {}
+                rest, seen = [], set()
+                for kind, sid, payload, fut in self._pending:   # one request per (session, kind) per tick, in arrival order
+                    if (sid, kind[0]) in seen:
+                        rest.append((kind, sid, payload, fut))
+                    else:
+                        seen.add((sid, kind[0]))
+                        batches.setdefault(kind, []).append((sid, payload, fut))
                 self._pending = rest
-            try:
-                res = self.tokenize_audio({sid: chunk for sid, chunk, _ in batch})
-                for sid, _, fut in batch:
-                    fut.set_result(res[sid])
-            except (ValueError, KeyError):
-                # a malformed request (bad chunk length, closed session) is rejected BEFORE anything is pushed: serve the
-                # others, fail only the offender
-                for sid, chunk, fut in batch:
-                    try:
-                        fut.set_result(self.tokenize_audio({sid: chunk})[sid])
-                    except Exception as ex:                # noqa: BLE001
-                        fut.set_exception(ex)
-            except Exception as ex:                        # noqa: BLE001  (engine failure: state unknown, everyone hears about it)
-                for _, _, fut in batch:
-                    if not fut.done():
-                        fut.set_exception(ex)
+            self._serve(self.tokenize_audio, batches.pop(("encode",), []))
+            for kind in sorted(k for k in batches if k[0] == "decode"):
+                self._serve(lambda reqs, pre=kind[1]: self.detokenize_audio(reqs, preroll_samples=pre), batches[kind])
+            self._serve(self.emit_output_chunks, batches.get(("emit",), []))
+
+    @staticmethod
+    def _serve(call, batch: List[Tuple[int, object, Future]]) -> None:
+        if not batch:
+            return
+        try:
+            res = call({sid: payload for sid, payload, _ in batch})
+            for sid, _, fut in batch:
+                fut.set_result(res[sid])
+        except (ValueError, KeyError):
+            # a malformed request (bad chunk length or string, closed session, emit not armed) is rejected BEFORE anything
+            # is pushed: serve the others, fail only the offender
+            for sid, payload, fut in batch:
+                try:
+                    fut.set_result(call({sid: payload})[sid])
+                except Exception as ex:                    # noqa: BLE001
+                    fut.set_exception(ex)
+        except Exception as ex:                            # noqa: BLE001  (engine failure: state unknown, everyone in the batch hears about it)
+            for _, _, fut in batch:
+                if not fut.done():
+                    fut.set_exception(ex)
