@@ -217,7 +217,9 @@ int mc_profile_end(mc_handle* h, double* ms, double* flops, double* bytes, int64
  * single pass of the convolution stack (bit-identical results; 0 recomputes it per window, for A/B tests);
  * "gemm_pair" — cta_group::2 GEMM where the shape allows; "fast_epilogue" — its mode-specialised epilogues
  * (bit-identical to the generic one); "attn_p_tmem" — attention keeps P in tensor memory (0: the shared-memory-P
- * kernel, bit-identical); "pdl" — programmatic dependent launch between the kernels of a pass. */
+ * kernel, bit-identical); "pdl" — programmatic dependent launch between the kernels of a pass; "exact_cut" — the
+ * transformer layers drop rows no kept output depends on at the exact row (0: only in steps of 16 frames, the earlier
+ * plan; bit-identical). */
 int mc_set_option(mc_handle* h, const char* key, int32_t value);
 /* impl: 0 = tensor-core kernels (default), 1 = SIMT cross-check kernels for attention / VQ; attention also
  * 2 = one-item-per-CTA tcgen05 kernel, 3 = two-slot persistent kernel without staged loads (A/B timing);
@@ -238,9 +240,11 @@ int mc_op_gemm(mc_handle* h, const void* A, int64_t a_rows, int32_t a_k_wrap, co
                int32_t rope_period, int32_t block_n, mc_stream_t stream);
 int mc_op_rmsnorm(mc_handle* h, const float* x, const float* gamma, void* out_bf16, int32_t M, int32_t d,
                   mc_stream_t stream);
-/* qkv bf16 [B*F, 3*d] (RoPE applied) -> out bf16 [B*F, d]. */
-int mc_op_attention(mc_handle* h, const void* qkv, void* out, int32_t B, int32_t F, int32_t impl,
-                    mc_stream_t stream);
+/* qkv bf16 [B*F, 3*d] (RoPE applied) -> out bf16 [B*out_rows, d]: the last out_rows queries of every window.
+ * phase (0 .. 15): the window is the tail of a longer one, (F_full - F) mod 16 frames past a 16-frame boundary; the
+ * tensor-core kernels then sum keys in the same groups as the full window, bit for bit.  0 for a whole window. */
+int mc_op_attention(mc_handle* h, const void* qkv, void* out, int32_t B, int32_t F, int32_t out_rows, int32_t phase,
+                    int32_t impl, mc_stream_t stream);
 
 /* The two kernels behind mc_stream_push_codes_emit / mc_embed_distance on caller-supplied DEVICE buffers
  * (the golden-vector replays of tests/test_gpu_post.py): wav [n_have], fade_in / prev_tail [fade] (prev_tail is

@@ -85,7 +85,7 @@ SYMBOLS = {
     "mc_op_gemm_fused": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I32, _I32, _I32, _P, _P, _I32, _P, _P, _P, _I32, _I32, _I32, _P]),
     "mc_op_rowstats": (C.c_int, [_P, _P, _P, _P, _P, _I32, _I32, _P]),
     "mc_op_rmsnorm": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _P]),
-    "mc_op_attention": (C.c_int, [_P, _P, _P, _I32, _I32, _I32, _P]),
+    "mc_op_attention": (C.c_int, [_P, _P, _P, _I32, _I32, _I32, _I32, _I32, _P]),
 }
 
 _lib: Optional[C.CDLL] = None

@@ -29,6 +29,14 @@ inline bool attn_sm100_supported(int wl, int wr) { return wr == 0 && wl <= ATT_H
 // ascending key order, so results do not depend on where a window was cut for dead-output elimination (adding the exact
 // zeros of masked keys is a no-op); P*V sums keys in 16-key UMMA groups.
 //
+// ATTENTION CUTS.  The row sum adds keys in pairs and P*V in 16-key groups, both counted from the first column of the
+// tile, so a frame must land at the same column mod 16 as in the full-window pass.  A window that dead-output
+// elimination cut to its last F rows (F_full - F frames dropped) is therefore laid out with phase = (F_full - F) mod 16
+// extra rows in front: Q and K/V tiles start `phase` rows before the window, i.e. at the previous window's last rows
+// (finite values written by the same QKV GEMM) or, for the first window, in TMA's out-of-bounds zero fill.  Those
+// columns are masked like any key before frame 0, and those query rows are never stored.  Every kept row then sees the
+// same key groups, in the same order, with the same values as in the full pass: results are bit-identical at any cut.
+//
 // =============================================================================================
 
 // v3: v2 with the operand loads decoupled from the compute slots.
@@ -77,7 +85,7 @@ template <int NKV>
 __global__ void __launch_bounds__(Att3Cfg<NKV>::kThreads, 1)
 attention_window_sm100_v3_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_kv,
                                  __nv_bfloat16* __restrict__ out, int B, int F, int H, int wl, int out_rows,
-                                 float scale_log2e) {
+                                 int phase, float scale_log2e) {
   using Cfg = Att3Cfg<NKV>;
   constexpr int NST = Cfg::kStages;
   constexpr int NSL = Cfg::kSlots;
@@ -96,8 +104,9 @@ attention_window_sm100_v3_kernel(const __grid_constant__ CUtensorMap map_q, cons
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int d = H * 64;
-  const int first_out = F - out_rows;
-  const int q_tiles = (F + ATT_BQ - 1) / ATT_BQ;
+  const int Fp = F + phase;   // tile layout of a window: `phase` masked rows in front of its F rows (see ATTENTION CUTS)
+  const int first_out = Fp - out_rows;
+  const int q_tiles = (Fp + ATT_BQ - 1) / ATT_BQ;
   const int first_tile = first_out / ATT_BQ;
   const int kept_tiles = q_tiles - first_tile;
   const int n_items = B * H * kept_tiles;
@@ -145,7 +154,7 @@ attention_window_sm100_v3_kernel(const __grid_constant__ CUtensorMap map_q, cons
         uint8_t* stage = smem + st * Cfg::kStageBytes;
         mbar_wait(&kv_free[st], use ^ 1);
         mbar_arrive_expect_tx(&kv_full[st], Cfg::kStageBytes);
-        const int row_q = b * F + qt * ATT_BQ;
+        const int row_q = b * F - phase + qt * ATT_BQ;
         tma_load_2d(stage, &map_q, &kv_full[st], h * 64, row_q);
         tma_load_2d(stage + ATT_SMEM_Q, &map_kv, &kv_full[st], d + h * 64, row_q - Cfg::kHalo);
         tma_load_2d(stage + ATT_SMEM_Q + NKV * 128, &map_kv, &kv_full[st], 2 * d + h * 64, row_q - Cfg::kHalo);
@@ -237,8 +246,8 @@ attention_window_sm100_v3_kernel(const __grid_constant__ CUtensorMap map_q, cons
       if (col_base >= 0) tmem_ld_32x32b_x32(tmem_s + lane_addr + col_base, raw0);
       tmem_ld_32x32b_x32(tmem_s + lane_addr + col_base + 32, raw1);
       tmem_ld_wait();
-      const int c_lo = max(r + Cfg::kHalo - wl, Cfg::kHalo - q0) - col_base;   // relative to col_base
-      const int c_hi = (qi < F) ? (r + Cfg::kHalo - col_base) : -1;
+      const int c_lo = max(r + Cfg::kHalo - wl, Cfg::kHalo - q0 + phase) - col_base;   // relative to col_base
+      const int c_hi = (qi < Fp) ? (r + Cfg::kHalo - col_base) : -1;
       float sc[64];
       float mx = -INFINITY;
 #pragma unroll
@@ -286,7 +295,7 @@ attention_window_sm100_v3_kernel(const __grid_constant__ CUtensorMap map_q, cons
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&slot_free[s]);   // S and O of this slot may be overwritten
-      if (qi < F && qi >= first_out) {
+      if (qi < Fp && qi >= first_out) {
         const float inv = 1.0f / sum;
         __nv_bfloat16* o = out + (static_cast<long long>(b) * out_rows + (qi - first_out)) * d + h * 64;
 #pragma unroll
@@ -341,7 +350,7 @@ template <int NKV>
 __global__ void __launch_bounds__(Att4Cfg<NKV>::kThreads, 1)
 attention_window_sm100_v4_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_kv,
                                  __nv_bfloat16* __restrict__ out, int B, int F, int H, int wl, int out_rows,
-                                 float scale_log2e) {
+                                 int phase, float scale_log2e) {
   using Cfg = Att4Cfg<NKV>;
   constexpr int NST = Cfg::kStages;
   constexpr int NSL = Cfg::kSlots;
@@ -359,8 +368,9 @@ attention_window_sm100_v4_kernel(const __grid_constant__ CUtensorMap map_q, cons
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int d = H * 64;
-  const int first_out = F - out_rows;
-  const int q_tiles = (F + ATT_BQ - 1) / ATT_BQ;
+  const int Fp = F + phase;   // tile layout of a window: `phase` masked rows in front of its F rows (see ATTENTION CUTS)
+  const int first_out = Fp - out_rows;
+  const int q_tiles = (Fp + ATT_BQ - 1) / ATT_BQ;
   const int first_tile = first_out / ATT_BQ;
   const int kept_tiles = q_tiles - first_tile;
   const int n_items = B * H * kept_tiles;
@@ -404,7 +414,7 @@ attention_window_sm100_v4_kernel(const __grid_constant__ CUtensorMap map_q, cons
         uint8_t* stage = smem + st * Cfg::kStageBytes;
         mbar_wait(&kv_free[st], use ^ 1);
         mbar_arrive_expect_tx(&kv_full[st], Cfg::kStageBytes);
-        const int row_q = b * F + qt * ATT_BQ;
+        const int row_q = b * F - phase + qt * ATT_BQ;
         tma_load_2d(stage, &map_q, &kv_full[st], h * 64, row_q);
         tma_load_2d(stage + ATT_SMEM_Q, &map_kv, &kv_full[st], d + h * 64, row_q - Cfg::kHalo);
         tma_load_2d(stage + ATT_SMEM_Q + NKV * 128, &map_kv, &kv_full[st], 2 * d + h * 64, row_q - Cfg::kHalo);
@@ -495,8 +505,8 @@ attention_window_sm100_v4_kernel(const __grid_constant__ CUtensorMap map_q, cons
       if (col_base >= 0) tmem_ld_32x32b_x32(tmem_s + lane_addr + col_base, raw0);
       tmem_ld_32x32b_x32(tmem_s + lane_addr + col_base + 32, raw1);
       tmem_ld_wait();
-      const int c_lo = max(r + Cfg::kHalo - wl, Cfg::kHalo - q0) - col_base;   // relative to col_base
-      const int c_hi = (qi < F) ? (r + Cfg::kHalo - col_base) : -1;
+      const int c_lo = max(r + Cfg::kHalo - wl, Cfg::kHalo - q0 + phase) - col_base;   // relative to col_base
+      const int c_hi = (qi < Fp) ? (r + Cfg::kHalo - col_base) : -1;
       float sc[64];
       float mx = -INFINITY;
 #pragma unroll
@@ -553,7 +563,7 @@ attention_window_sm100_v4_kernel(const __grid_constant__ CUtensorMap map_q, cons
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&slot_free[s]);   // S and O of this slot may be overwritten
-      if (qi < F && qi >= first_out) {
+      if (qi < Fp && qi >= first_out) {
         const float inv = 1.0f / sum;
         __nv_bfloat16* o = out + (static_cast<long long>(b) * out_rows + (qi - first_out)) * d + h * 64;
 #pragma unroll
@@ -588,7 +598,7 @@ attention_window_sm100_v4_kernel(const __grid_constant__ CUtensorMap map_q, cons
 
 template <int NKV>
 inline int launch_attention_sm100_v4_nkv(mc_handle* h, const bf16* qkv, bf16* out, int B, int F, int out_rows,
-                                         cudaStream_t stream) {
+                                         int phase, cudaStream_t stream) {
   using Cfg = Att4Cfg<NKV>;
   const mc_spec& s = h->spec;
   const int d = s.d_model;
@@ -596,19 +606,19 @@ inline int launch_attention_sm100_v4_nkv(mc_handle* h, const bf16* qkv, bf16* ou
   MC_TRY(mc_internal::get_map_2d_bf16(h, qkv, (uint64_t)3 * d, (uint64_t)B * F, 64, ATT_BQ, &mq));
   MC_TRY(mc_internal::get_map_2d_bf16(h, qkv, (uint64_t)3 * d, (uint64_t)B * F, 64, NKV, &mkv));
   MC_TRY(mc_allow_smem(h, attention_window_sm100_v4_kernel<NKV>, Cfg::kSmemBytes));
-  const int q_tiles = (F + ATT_BQ - 1) / ATT_BQ;
-  const long long items = (long long)B * s.n_heads * (q_tiles - (F - out_rows) / ATT_BQ);
+  const int q_tiles = (F + phase + ATT_BQ - 1) / ATT_BQ;
+  const long long items = (long long)B * s.n_heads * (q_tiles - (F + phase - out_rows) / ATT_BQ);
   if (items > INT_MAX) return h->fail(MC_ERR_ARG, "attention: too many tiles");
   const int grid = (int)std::min<long long>(items, h->num_sms);
   mc_launch(h, attention_window_sm100_v4_kernel<NKV>, dim3(grid), dim3(Cfg::kThreads), Cfg::kSmemBytes, stream, *mq, *mkv, out, B, F,
-            s.n_heads, s.window_left, out_rows, 0.125f * 1.4426950408889634f);
+            s.n_heads, s.window_left, out_rows, phase, 0.125f * 1.4426950408889634f);
   MC_LAUNCH_CHECK(h, "attention_window_sm100_v4_kernel");
   return MC_OK;
 }
 
 template <int NKV>
 inline int launch_attention_sm100_v3_nkv(mc_handle* h, const bf16* qkv, bf16* out, int B, int F, int out_rows,
-                                         cudaStream_t stream) {
+                                         int phase, cudaStream_t stream) {
   using Cfg = Att3Cfg<NKV>;
   const mc_spec& s = h->spec;
   const int d = s.d_model;
@@ -616,24 +626,27 @@ inline int launch_attention_sm100_v3_nkv(mc_handle* h, const bf16* qkv, bf16* ou
   MC_TRY(mc_internal::get_map_2d_bf16(h, qkv, (uint64_t)3 * d, (uint64_t)B * F, 64, ATT_BQ, &mq));
   MC_TRY(mc_internal::get_map_2d_bf16(h, qkv, (uint64_t)3 * d, (uint64_t)B * F, 64, NKV, &mkv));
   MC_TRY(mc_allow_smem(h, attention_window_sm100_v3_kernel<NKV>, Cfg::kSmemBytes));
-  const int q_tiles = (F + ATT_BQ - 1) / ATT_BQ;
-  const long long items = (long long)B * s.n_heads * (q_tiles - (F - out_rows) / ATT_BQ);
+  const int q_tiles = (F + phase + ATT_BQ - 1) / ATT_BQ;
+  const long long items = (long long)B * s.n_heads * (q_tiles - (F + phase - out_rows) / ATT_BQ);
   if (items > INT_MAX) return h->fail(MC_ERR_ARG, "attention: too many tiles");
   const int grid = (int)std::min<long long>(items, h->num_sms);
   mc_launch(h, attention_window_sm100_v3_kernel<NKV>, dim3(grid), dim3(Cfg::kThreads), Cfg::kSmemBytes, stream, *mq, *mkv, out, B, F,
-            s.n_heads, s.window_left, out_rows, 0.125f * 1.4426950408889634f);
+            s.n_heads, s.window_left, out_rows, phase, 0.125f * 1.4426950408889634f);
   MC_LAUNCH_CHECK(h, "attention_window_sm100_v3_kernel");
   return MC_OK;
 }
 
-inline int launch_attention_sm100_v3(mc_handle* h, const bf16* qkv, bf16* out, int B, int F, int out_rows,
+// phase: rows in front of the window that complete its first 16-key group (0 .. 15; see ATTENTION CUTS)
+inline int launch_attention_sm100_v3(mc_handle* h, const bf16* qkv, bf16* out, int B, int F, int out_rows, int phase,
                                      cudaStream_t stream) {
+  if (phase < 0 || phase > 15) return h->fail(MC_ERR_ARG, "attention: cut phase %d is not in 0 .. 15", phase);
+  const bool one_tile = F + phase <= ATT_BQ;
   if (h->attn_p_tmem) {
-    if (F <= ATT_BQ) return launch_attention_sm100_v4_nkv<128>(h, qkv, out, B, F, out_rows, stream);
-    return launch_attention_sm100_v4_nkv<160>(h, qkv, out, B, F, out_rows, stream);
+    if (one_tile) return launch_attention_sm100_v4_nkv<128>(h, qkv, out, B, F, out_rows, phase, stream);
+    return launch_attention_sm100_v4_nkv<160>(h, qkv, out, B, F, out_rows, phase, stream);
   }
-  if (F <= ATT_BQ) return launch_attention_sm100_v3_nkv<128>(h, qkv, out, B, F, out_rows, stream);
-  return launch_attention_sm100_v3_nkv<160>(h, qkv, out, B, F, out_rows, stream);
+  if (one_tile) return launch_attention_sm100_v3_nkv<128>(h, qkv, out, B, F, out_rows, phase, stream);
+  return launch_attention_sm100_v3_nkv<160>(h, qkv, out, B, F, out_rows, phase, stream);
 }
 
 }  // namespace mc

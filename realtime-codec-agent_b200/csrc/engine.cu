@@ -266,14 +266,17 @@ int launch_rmsnorm(mc_handle* h, const float* x, const float* gamma, bf16* out, 
   return MC_OK;
 }
 
-// qkv [B*F, 3d] -> out [B*out_rows, d]: only the last out_rows queries of each window are kept
-int launch_attention(mc_handle* h, const bf16* qkv, bf16* out, int B, int F, int out_rows, int impl, cudaStream_t stream) {
+// qkv [B*F, 3d] -> out [B*out_rows, d]: only the last out_rows queries of each window are kept.  phase (0 .. 15) places a
+// window cut from a longer one on the key groups of the full-window pass (attn_sm100.cuh, ATTENTION CUTS); the SIMT
+// kernel sums every row's keys from its own first key, so it is cut-invariant already and ignores it.
+int launch_attention(mc_handle* h, const bf16* qkv, bf16* out, int B, int F, int out_rows, int phase, int impl, cudaStream_t stream) {
+  if (out_rows < 1 || out_rows > F) return h->fail(MC_ERR_ARG, "attention: out_rows %d not in 1 .. %d", out_rows, F);
   const mc_spec& s = h->spec;
   const double span = std::min(F, s.window_left + s.window_right + 1);
   McProfScope prof(h, 1, 4.0 * B * out_rows * span * s.d_model,
                    (double)B * (F * 2.0 + out_rows * 2.0) * s.d_model * 2.0, stream);
   if (impl == 0 && attn_sm100_supported(s.window_left, s.window_right)) {   // v4 (P in tensor memory) or, with attn_p_tmem = 0, v3
-    MC_TRY(launch_attention_sm100_v3(h, qkv, out, B, F, out_rows, stream));
+    MC_TRY(launch_attention_sm100_v3(h, qkv, out, B, F, out_rows, phase, stream));
     return MC_OK;
   }
   if (impl != 0 && impl != 1) return h->fail(MC_ERR_ARG, "attention: unknown implementation %d (0 = tcgen05, 1 = SIMT cross-check)", impl);
@@ -324,7 +327,8 @@ int launch_rowstats(mc_handle* h, const float* x, const float* gamma, bf16* xb, 
 // Dead-output elimination (exact): a layer whose output is needed only for the last R_out rows
 // needs keys/values for the last R_in = min(F, R_out + window_left) rows, so working backwards from
 // keep_rows each layer gets (R_in, R_out); rows outside are never computed.  Per-row arithmetic is
-// unchanged (same K order, same epilogues), so kept rows are bit-identical to the full pass.
+// unchanged (same K order, same epilogues), and attention lays a cut window out on the full pass's
+// 16-key groups (phase = (F - R_in) mod 16, attn_sm100.cuh), so kept rows are bit-identical to the full pass.
 //
 // fused = true (few-rows path): the caller has already put bf16(x * gamma_norm1[0]) in b.hbuf and the rows' partial sums
 // of squares in b.stats (its last GEMM ran as a "producer"); every norm of the stack then lives in GEMM epilogues — QKV
@@ -349,10 +353,8 @@ int run_layers(mc_handle* h, const char* prefix, int n_layers, const StackBufs& 
     for (int l = n_layers - 1; l >= 0; --l) {
       r_out[l] = need;
       need = (need >= F) ? F : std::min(F, need + s.window_left);
-      // Cut windows only at multiples of 16 frames: the P*V UMMA sums keys in groups of 16, and a cut
-      // that shifts a row's keys relative to those groups would change the summation order (results
-      // would still be correct but no longer bit-identical to the full-window pass).
-      if (need < F) need = F - ((F - need) / 16) * 16;
+      // exact_cut = 0: the earlier plan, which cut windows only at multiples of 16 frames (kept for A/B runs)
+      if (!h->exact_cut && need < F) need = F - ((F - need) / 16) * 16;
       r_in[l] = need;
     }
   }
@@ -375,7 +377,7 @@ int run_layers(mc_handle* h, const char* prefix, int n_layers, const StackBufs& 
     g.rope_cols = 2 * d; g.rope_period = Ri; g.rope_offset = F - Ri;
     g.prefetch_ptr = h->ptr<bf16>(T("wo")); g.prefetch_bytes = (long long)d * d * 2;
     MC_TRY(launch_gemm(h, g, stream));
-    MC_TRY(launch_attention(h, b.qkv, b.att, B, Ri, Ro, h->attn_impl, stream));
+    MC_TRY(launch_attention(h, b.qkv, b.att, B, Ri, Ro, (F - Ri) % 16, h->attn_impl, stream));
     if (Ro < Ri) {
       const long long items = (long long)Mo * (d / 4);
       McProfScope prof(h, 3, 0.0, (double)Mo * d * 8.0, stream);
@@ -1041,6 +1043,7 @@ int mc_set_option(mc_handle* h, const char* key, int32_t value) {
   if (!h || !key) return MC_ERR_ARG;
   const std::string k(key);
   if (k == "shared_stem") h->shared_stem = value != 0;
+  else if (k == "exact_cut") { h->exact_cut = value != 0; h->tensor_gen++; }
   else if (k == "gemm_pair") h->gemm_pair = value != 0;
   else if (k == "fast_epilogue") h->fast_epilogue = value != 0;
   else if (k == "pdl") h->pdl = value != 0;
@@ -1121,11 +1124,13 @@ int mc_op_rmsnorm(mc_handle* h, const float* x, const float* gamma, void* out_bf
   return launch_rmsnorm(h, x, gamma, reinterpret_cast<bf16*>(out_bf16), M, d, INT_MAX, 0, 0, (cudaStream_t)stream);
 }
 
-int mc_op_attention(mc_handle* h, const void* qkv, void* out, int32_t B, int32_t F, int32_t impl, mc_stream_t stream) {
+int mc_op_attention(mc_handle* h, const void* qkv, void* out, int32_t B, int32_t F, int32_t out_rows, int32_t phase,
+                    int32_t impl, mc_stream_t stream) {
   MC_ENTER(h);
   for (int r = 1; r < h->debug_repeat; ++r)
-    MC_TRY(launch_attention(h, reinterpret_cast<const bf16*>(qkv), reinterpret_cast<bf16*>(out), B, F, F, impl, (cudaStream_t)stream));
-  return launch_attention(h, reinterpret_cast<const bf16*>(qkv), reinterpret_cast<bf16*>(out), B, F, F, impl,
+    MC_TRY(launch_attention(h, reinterpret_cast<const bf16*>(qkv), reinterpret_cast<bf16*>(out), B, F, out_rows, phase, impl,
+                            (cudaStream_t)stream));
+  return launch_attention(h, reinterpret_cast<const bf16*>(qkv), reinterpret_cast<bf16*>(out), B, F, out_rows, phase, impl,
                           (cudaStream_t)stream);
 }
 

@@ -73,6 +73,7 @@ struct mc_handle {
   bool l2_prefetch = true;    // split-K GEMMs pull the next GEMM's weights into L2 while they run
   bool pdl = true;            // programmatic dependent launch between consecutive kernels of a pass
   bool shared_stem = true;  // overlapping hop-aligned windows share one pass of the conv stack (exact)
+  bool exact_cut = true;    // dead-output elimination cuts windows at the exact row, not at multiples of 16 frames (exact)
   // optional per-class device timing (bench.py's roofline): event pairs around each launch
   struct ProfRec { cudaEvent_t a, b; int cls; double flops; double bytes; };
   bool profiling = false;

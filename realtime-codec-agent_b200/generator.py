@@ -607,8 +607,10 @@ class B200Generator:
         nat.check(self._lib, self._handle, rc, "mc_op_rmsnorm")
         return out
 
-    def op_attention(self, qkv, B, F, impl=0):
-        out = torch.empty((B * F, self.spec.d_model), dtype=BF16, device=self.device)
-        rc = self._lib.mc_op_attention(self._handle, qkv.data_ptr(), out.data_ptr(), B, F, impl, self._stream())
+    def op_attention(self, qkv, B, F, impl=0, out_rows=None, phase=0):
+        out_rows = F if out_rows is None else out_rows
+        out = torch.empty((B * out_rows, self.spec.d_model), dtype=BF16, device=self.device)
+        rc = self._lib.mc_op_attention(self._handle, qkv.data_ptr(), out.data_ptr(), B, F, out_rows, phase, impl,
+                                       self._stream())
         nat.check(self._lib, self._handle, rc, "mc_op_attention")
         return out
