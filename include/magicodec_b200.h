@@ -199,6 +199,28 @@ int mc_pool_set_emit(mc_pool* p, int32_t chunk_samples, int32_t fade_samples, fl
 int mc_pool_push_codes_emit(mc_pool* p, const int32_t* slots, int32_t n, const int64_t* codes, int32_t len, float* out,
                             int32_t* had_prev, mc_stream_t stream);
 
+/* ---- ragged pool calls: the same per-session semantics, but the sessions of one call may hold contexts of different
+ * length (streams in their warm-up next to streams in steady state), in ONE launch.  Every window starts at row 0 of
+ * the batch and reads zeros (codes: code 0) past its own end; the codec is causal for window_right == 0, so each
+ * session's kept frames equal its lone pass (bit for bit with small_m_split_k = 0).  Equal lengths take the uniform
+ * call (same results, same graphs); different lengths on a spec with window_right != 0 fail with MC_ERR_ARG.  Every
+ * check runs before any work or state change.
+ * push_audio_ragged: 1 <= keep_frames <= ceil(len / hop); codes_out HOST int64 [n][C][keep_frames], item j = the last
+ *   keep_frames frames of its own window.
+ * push_codes_ragged: 1 <= keep_samples <= ceil(capacity / hop) * hop; item j gets min(keep_samples, new_len_j * hop) samples,
+ *   the last ones of its window, at the start of its wav_out row HOST fp32 [n][C][keep_samples] (zeros after them);
+ *   samples_out HOST int32 [n] = that count per item.
+ * push_codes_emit_ragged: mc_pool_push_codes_emit where first chunks may mix with continuing ones; the rules of
+ *   mc_pool_push_codes_emit hold per item; had_prev HOST int32 [n].
+ * graph_count: distinct graph keys seen and graphs captured (all push calls of the pool). */
+int mc_pool_push_audio_ragged(mc_pool* p, const int32_t* slots, int32_t n, const float* chunks, int32_t len, int32_t keep_frames,
+                              int64_t* codes_out, mc_stream_t stream);
+int mc_pool_push_codes_ragged(mc_pool* p, const int32_t* slots, int32_t n, const int64_t* codes, int32_t len, int32_t keep_samples,
+                              float* wav_out, int32_t* samples_out, mc_stream_t stream);
+int mc_pool_push_codes_emit_ragged(mc_pool* p, const int32_t* slots, int32_t n, const int64_t* codes, int32_t len, float* out,
+                                   int32_t* had_prev, mc_stream_t stream);
+int mc_pool_graph_count(mc_pool* p, int32_t* keys, int32_t* captured);
+
 /* ids DEVICE int64 [rows, n] (LM token ids; code = id - vocab_start, clamped to the codebook).
  * dist_out DEVICE fp32 [rows] (optional) = mean_j ||E[code_j] - ref||_2, ref DEVICE fp32 [dq] (NULL = 0);
  * mean_out DEVICE fp32 [rows, dq] (optional) = mean_j E[code_j], E = the cached projected codebook. */

@@ -71,6 +71,10 @@ SYMBOLS = {
     "mc_pool_push_codes": (C.c_int, [_P, _P, _I32, _P, _I32, _I32, _P, C.POINTER(_I32), _P]),
     "mc_pool_set_emit": (C.c_int, [_P, _I32, _I32, C.c_float, C.c_float, _P]),
     "mc_pool_push_codes_emit": (C.c_int, [_P, _P, _I32, _P, _I32, _P, C.POINTER(_I32), _P]),
+    "mc_pool_push_audio_ragged": (C.c_int, [_P, _P, _I32, _P, _I32, _I32, _P, _P]),
+    "mc_pool_push_codes_ragged": (C.c_int, [_P, _P, _I32, _P, _I32, _I32, _P, _P, _P]),
+    "mc_pool_push_codes_emit_ragged": (C.c_int, [_P, _P, _I32, _P, _I32, _P, _P, _P]),
+    "mc_pool_graph_count": (C.c_int, [_P, C.POINTER(_I32), C.POINTER(_I32)]),
     "mc_embed_distance": (C.c_int, [_P, _P, _I32, _I32, _I64, _P, _P, _P, _P]),
     "mc_op_gemm": (C.c_int, [_P, _P, _I64, _I32, _P, _P, _I32, _I32, _I32, _I32, _I32, _P, _I64,
                              _I32, _I32, _I64, _I64, _I32, _I32, _I32, _P]),

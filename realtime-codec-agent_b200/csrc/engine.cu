@@ -563,8 +563,15 @@ int stem_prefix_frames(const mc_spec& s) {
   return (int)dirty;
 }
 
+// A ragged session-pool batch (mc_pool_push_audio_ragged): encode_impl's `keep` rows of every window run through the
+// stack, then each item's own last `keep` frames (rtable: pool_roll_ragged_kernel's table) are gathered for the VQ.
+struct RaggedKeep {
+  const int* rtable;
+  int C, keep;
+};
+
 int encode_impl(mc_handle* h, const float* wav, int64_t ld, int B, int T, int keep, int64_t* codes, float* margin,
-                float* z_e_out, cudaStream_t stream) {
+                float* z_e_out, cudaStream_t stream, const RaggedKeep* ragged = nullptr) {
   const mc_spec& s = h->spec;
   const int n = s.n_convs;
   int hop = 1;
@@ -609,6 +616,7 @@ int encode_impl(mc_handle* h, const float* wav, int64_t ld, int B, int T, int ke
   carve_stack(cv2, nullptr, M, d, s.ffn_dim, true);
   size_t oz = cv2.take((size_t)M * dq * 4);
   size_t ovq = cv2.take(vq_scratch_bytes(h, B * keep));
+  const size_t ozg = ragged ? cv2.take((size_t)B * ragged->keep * dq * 4) : 0;
   MC_TRY(arena_reserve(h, cv2.off, stream));
   uint8_t* base = h->arena;
   StackBufs sb = carve_stack(cv, base, M, d, s.ffn_dim, false);
@@ -647,6 +655,13 @@ int encode_impl(mc_handle* h, const float* wav, int64_t ld, int B, int T, int ke
   MC_TRY(launch_gemm(h, pj, stream));
   if (z_e_out) MC_CUDA(h, cudaMemcpyAsync(z_e_out, z_e, (size_t)M * dq * 4, cudaMemcpyDeviceToDevice, stream));
   // ---- quantise the kept frames (z_e holds keep_rows rows per window)
+  if (ragged) {
+    float* zg = reinterpret_cast<float*>(base + ozg);
+    pool_gather_rows_ragged_kernel<<<dim3(1, B), 256, 0, stream>>>(z_e, ragged->rtable, ragged->C, keep_rows, F, ragged->keep,
+                                                                   dq, hop, zg);
+    MC_LAUNCH_CHECK(h, "pool_gather_rows_ragged_kernel");
+    return launch_vq(h, zg, B, ragged->keep, ragged->keep, codes, margin, vq_scratch, stream);
+  }
   MC_TRY(launch_vq(h, z_e, B, keep_rows, keep, codes, margin, vq_scratch, stream));
   return MC_OK;
 }
@@ -1190,20 +1205,20 @@ void stream_drop_graphs(mc_stream* s) {
 
 // Runs `body` directly the first time a key is seen (that run sizes the workspace and fills the TMA
 // descriptor cache), captures it into a graph the second time, and replays the graph afterwards.
-template <typename Sess, typename Body>
-int run_or_replay_impl(Sess* s, std::tuple<int, int, int, int, int> key, cudaStream_t stream, Body body);
+template <typename Sess, typename Key, typename Body>
+int run_or_replay_impl(Sess* s, Key key, cudaStream_t stream, Body body);
 
 // Everything a session launches (directly or while capturing) is "in session": few-rows GEMMs take the split-K kernels.
-template <typename Sess, typename Body>
-int run_or_replay(Sess* s, std::tuple<int, int, int, int, int> key, cudaStream_t stream, Body body) {
+template <typename Sess, typename Key, typename Body>
+int run_or_replay(Sess* s, Key key, cudaStream_t stream, Body body) {
   s->h->in_session = true;
   const int rc = run_or_replay_impl(s, key, stream, body);
   s->h->in_session = false;
   return rc;
 }
 
-template <typename Sess, typename Body>
-int run_or_replay_impl(Sess* s, std::tuple<int, int, int, int, int> key, cudaStream_t stream, Body body) {
+template <typename Sess, typename Key, typename Body>
+int run_or_replay_impl(Sess* s, Key key, cudaStream_t stream, Body body) {
   mc_handle* h = s->h;
   if (!s->use_graphs || h->profiling) return body();
   auto& e = s->graphs[key];
@@ -1526,11 +1541,13 @@ struct mc_pool {
   std::vector<int> audio_len, code_len, acur, ccur;
   float *pin_chunk = nullptr, *dev_chunk = nullptr, *batch_audio = nullptr;          // [max_sessions*C][cap_samples]
   int64_t *pin_codes_in = nullptr, *dev_codes_in = nullptr, *batch_codes = nullptr;  // [max_sessions*C][cap_frames]
-  int32_t *pin_table = nullptr, *dev_table = nullptr;                                // [max_sessions][2]
+  int32_t *pin_table = nullptr, *dev_table = nullptr;                                // [max_sessions][2], ragged [max_sessions][4]
   int64_t *dev_codes_out = nullptr, *pin_codes_out = nullptr;
   float *dev_wav_out = nullptr, *pin_wav_out = nullptr;
   struct GraphEntry { cudaGraphExec_t exec = nullptr; int uses = 0; size_t arena_gen = 0; };
-  std::map<std::tuple<int, int, int, int, int>, GraphEntry> graphs;   // (kind, len_before, n_new, keep, batch items)
+  // uniform calls: (kind 0-3, len_before, n_new, keep, batch items, 0); ragged calls: (kind 4-6, T_max or F_max, n_new,
+  // cut, batch items, keep) -- the per-item lengths live in the table the graph uploads
+  std::map<std::tuple<int, int, int, int, int, int>, GraphEntry> graphs;
   bool use_graphs = true;
   cudaStream_t own = nullptr;
   cudaEvent_t order_ev = nullptr;
@@ -1558,19 +1575,53 @@ void pool_free_emit(mc_pool* p) {
   p->emit_chunk = p->emit_fade = 0;
 }
 
-int pool_check_slots(mc_pool* p, const int32_t* slots, int n, const std::vector<int>& lens, int* common_len, const char* what) {
+// same_len = false (ragged calls): any context lengths; *common_len = -1 when they differ.
+int pool_check_slots(mc_pool* p, const int32_t* slots, int n, const std::vector<int>& lens, int* common_len, const char* what,
+                     bool same_len = true) {
   mc_handle* h = p->h;
   if (!slots || n < 1 || n > p->max_sessions) return h->fail(MC_ERR_ARG, "%s: need 1..%d sessions, got %d", what, p->max_sessions, n);
   for (int j = 0; j < n; ++j) {
     if (slots[j] < 0 || slots[j] >= p->max_sessions) return h->fail(MC_ERR_ARG, "%s: slot %d out of range", what, slots[j]);
     for (int k = 0; k < j; ++k)
       if (slots[k] == slots[j]) return h->fail(MC_ERR_ARG, "%s: slot %d listed twice", what, slots[j]);
-    if (lens[slots[j]] != lens[slots[0]])
+    if (same_len && lens[slots[j]] != lens[slots[0]])
       return h->fail(MC_ERR_ARG, "%s: sessions %d and %d hold contexts of different length (%d vs %d); batch them separately", what,
                      slots[0], slots[j], lens[slots[0]], lens[slots[j]]);
   }
   *common_len = lens[slots[0]];
+  for (int j = 1; j < n; ++j)
+    if (lens[slots[j]] != lens[slots[0]]) *common_len = -1;
   return MC_OK;
+}
+
+// Ragged calls: the pinned table of pool_roll_ragged_kernel, {slot, context buffer, old_len, new_len} per item, for
+// contexts that keep the last max(len, ctx) values; returns the longest new context.
+int pool_fill_ragged_table(mc_pool* p, const int32_t* slots, int n, int len, int ctx, const std::vector<int>& lens,
+                           const std::vector<int>& cur) {
+  int longest = 0;
+  for (int j = 0; j < n; ++j) {
+    const int s = slots[j], new_len = std::min(lens[s] + len, std::max(len, ctx));
+    int32_t* t = p->pin_table + 4 * j;
+    t[0] = s; t[1] = cur[s]; t[2] = lens[s]; t[3] = new_len;
+    longest = std::max(longest, new_len);
+  }
+  return longest;
+}
+
+// Rows of a ragged batch's last transformer layers: rounded up to 16 to bound the number of graphs (the cut is exact at
+// any depth), never more than the window.
+int ragged_cut(int rows, int F) { return std::min(F, (rows + 15) / 16 * 16); }
+
+// Decoder rows of a ragged decode whose items keep keep_j = min(keep, F_j * hop) samples each (the earliest kept sample
+// over the batch, plus the two frames the transposed convs look back), and the `keep` decode_impl takes for that cut.
+void ragged_decode_cut(const mc_pool* p, int n, int F_max, int hop, int keep, int* rows, int* dec_keep) {
+  int need = 0;
+  for (int j = 0; j < n; ++j) {
+    const int total_j = p->pin_table[4 * j + 3] * hop;
+    need = std::max(need, (F_max * hop - total_j) + std::min(keep, total_j));
+  }
+  *rows = ragged_cut((need + hop - 1) / hop + 2, F_max);
+  *dec_keep = *rows >= F_max ? F_max * hop : (*rows - 2) * hop;
 }
 }  // namespace
 
@@ -1610,16 +1661,17 @@ int mc_pool_create(mc_handle* h, int32_t channels, int32_t context_samples, int3
   p->emit_has_prev.assign(max_sessions, 0);
   const size_t rows = (size_t)max_sessions * channels;
   const size_t ab = rows * p->cap_samples * 4, cb = rows * p->cap_frames * 8;
+  const size_t wb = rows * p->cap_frames * hop * 4;   // decoded windows: up to cap_frames * hop >= cap_samples samples each
   cudaError_t e = cudaSuccess;
   auto dev = [&](void** q, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(q, bytes); };
   auto pin = [&](void** q, size_t bytes) { if (e == cudaSuccess) e = cudaMallocHost(q, bytes); };
   for (int i = 0; i < 2; ++i) { dev((void**)&p->audio[i], ab); dev((void**)&p->codes[i], cb); }
-  dev((void**)&p->dev_chunk, ab); dev((void**)&p->batch_audio, ab); dev((void**)&p->dev_wav_out, ab);
+  dev((void**)&p->dev_chunk, ab); dev((void**)&p->batch_audio, ab); dev((void**)&p->dev_wav_out, wb);
   dev((void**)&p->dev_codes_in, cb); dev((void**)&p->batch_codes, cb); dev((void**)&p->dev_codes_out, cb);
-  dev((void**)&p->dev_table, (size_t)max_sessions * 8);
-  pin((void**)&p->pin_chunk, ab); pin((void**)&p->pin_wav_out, ab);
+  dev((void**)&p->dev_table, (size_t)max_sessions * 16);
+  pin((void**)&p->pin_chunk, ab); pin((void**)&p->pin_wav_out, wb);
   pin((void**)&p->pin_codes_in, cb); pin((void**)&p->pin_codes_out, cb);
-  pin((void**)&p->pin_table, (size_t)max_sessions * 8);
+  pin((void**)&p->pin_table, (size_t)max_sessions * 16);
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->own, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p->order_ev, cudaEventDisableTiming);
   if (e != cudaSuccess) { mc_pool_destroy(p); return h->fail(MC_ERR_NOMEM, "mc_pool_create: %s", cudaGetErrorString(e)); }
@@ -1680,7 +1732,7 @@ int mc_pool_push_audio(mc_pool* p, const int32_t* slots, int32_t n, const float*
     MC_CUDA(h, cudaMemcpyAsync(p->pin_codes_out, p->dev_codes_out, (size_t)rows * keep * 8, cudaMemcpyDeviceToHost, stream));
     return MC_OK;
   };
-  MC_TRY(run_or_replay(p, std::make_tuple(0, old_len, len, keep, n), stream, body));
+  MC_TRY(run_or_replay(p, std::make_tuple(0, old_len, len, keep, n, 0), stream, body));
   MC_CUDA(h, cudaStreamSynchronize(stream));
   memcpy(codes_out, p->pin_codes_out, (size_t)rows * keep * 8);
   if (frames_out) *frames_out = keep;
@@ -1721,7 +1773,7 @@ int mc_pool_push_codes(mc_pool* p, const int32_t* slots, int32_t n, const int64_
     MC_CUDA(h, cudaMemcpyAsync(p->pin_wav_out, p->dev_wav_out, (size_t)rows * keep * 4, cudaMemcpyDeviceToHost, stream));
     return MC_OK;
   };
-  MC_TRY(run_or_replay(p, std::make_tuple(1, old_len, len, keep, n), stream, body));
+  MC_TRY(run_or_replay(p, std::make_tuple(1, old_len, len, keep, n, 0), stream, body));
   MC_CUDA(h, cudaStreamSynchronize(stream));
   memcpy(wav_out, p->pin_wav_out, (size_t)rows * keep * 4);
   if (samples_out) *samples_out = keep;
@@ -1811,11 +1863,200 @@ int mc_pool_push_codes_emit(mc_pool* p, const int32_t* slots, int32_t n, const i
     MC_LAUNCH_CHECK(h, "emit_chunk_pool_kernel");
     return MC_OK;
   };
-  MC_TRY(run_or_replay(p, std::make_tuple(2 + has_prev, old_len, len, keep, n), stream, body));
+  MC_TRY(run_or_replay(p, std::make_tuple(2 + has_prev, old_len, len, keep, n, 0), stream, body));
   MC_CUDA(h, cudaStreamSynchronize(stream));
   memcpy(out, p->pin_emit, (size_t)n * block * 4);
   if (had_prev) *had_prev = has_prev;
   for (int j = 0; j < n; ++j) { p->ccur[slots[j]] ^= 1; p->code_len[slots[j]] = new_len; p->emit_has_prev[slots[j]] = 1; }
+  return MC_OK;
+}
+
+// ---- ragged batches: the sessions of one call may hold contexts of different length (a stream in its warm-up next to
+// ones in steady state).  Equal lengths take the uniform call above; different lengths need causal attention.
+namespace {
+int pool_ragged_causal(mc_pool* p, const char* what) {
+  if (p->h->spec.window_right != 0)
+    return p->h->fail(MC_ERR_ARG, "%s: contexts of different length need causal attention (window_right = %d); batch them separately",
+                      what, p->h->spec.window_right);
+  return MC_OK;
+}
+}  // namespace
+
+int mc_pool_push_audio_ragged(mc_pool* p, const int32_t* slots, int32_t n, const float* chunks, int32_t len, int32_t keep_frames,
+                              int64_t* codes_out, mc_stream_t stream_) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  int common = 0;
+  MC_TRY(pool_check_slots(p, slots, n, p->audio_len, &common, "mc_pool_push_audio_ragged", false));
+  if (!chunks || !codes_out || len < 1) return h->fail(MC_ERR_ARG, "mc_pool_push_audio_ragged: bad arguments");
+  if (len > p->cap_samples)
+    return h->fail(MC_ERR_ARG, "mc_pool_push_audio_ragged: chunk of %d samples exceeds the capacity %d", len, p->cap_samples);
+  int hop = 1;
+  for (int i = 0; i < h->spec.n_convs; ++i) hop *= h->spec.conv_strides[i];
+  if (keep_frames < 1 || keep_frames > (len + hop - 1) / hop)
+    return h->fail(MC_ERR_ARG, "mc_pool_push_audio_ragged: keep_frames %d outside 1..%d", keep_frames, (len + hop - 1) / hop);
+  if (common >= 0) return mc_pool_push_audio(p, slots, n, chunks, len, keep_frames, codes_out, nullptr, stream_);
+  MC_TRY(pool_ragged_causal(p, "mc_pool_push_audio_ragged"));
+  MC_CUDA(h, cudaEventRecord(p->order_ev, (cudaStream_t)stream_));
+  MC_CUDA(h, cudaStreamWaitEvent(p->own, p->order_ev, 0));
+  cudaStream_t stream = p->own;
+  const int C = p->C, cap = p->cap_samples, rows = n * C, keep = keep_frames;
+  const int T_max = pool_fill_ragged_table(p, slots, n, len, p->ctx_samples, p->audio_len, p->acur);
+  const int F_max = (T_max + hop - 1) / hop;
+  int F_min = F_max;
+  for (int j = 0; j < n; ++j) F_min = std::min(F_min, (p->pin_table[4 * j + 3] + hop - 1) / hop);
+  const int cut = ragged_cut(F_max - F_min + keep, F_max);
+  for (int r = 0; r < rows; ++r) memcpy(p->pin_chunk + (size_t)r * cap, chunks + (size_t)r * len, (size_t)len * 4);
+  const RaggedKeep rg{p->dev_table, C, keep};
+  auto body = [&]() -> int {
+    MC_CUDA(h, cudaMemcpyAsync(p->dev_table, p->pin_table, (size_t)n * 16, cudaMemcpyHostToDevice, stream));
+    MC_CUDA(h, cudaMemcpy2DAsync(p->dev_chunk, (size_t)cap * 4, p->pin_chunk, (size_t)cap * 4, (size_t)len * 4, rows, cudaMemcpyHostToDevice, stream));
+    pool_roll_ragged_kernel<float><<<dim3((T_max + 255) / 256, rows), 256, 0, stream>>>(p->dev_table, C, cap, len, p->audio[0], p->audio[1],
+                                                                                       p->dev_chunk, p->batch_audio, cap, T_max);
+    MC_LAUNCH_CHECK(h, "pool_roll_ragged_kernel");
+    MC_TRY(encode_impl(h, p->batch_audio, cap, rows, T_max, cut, p->dev_codes_out, nullptr, nullptr, stream, &rg));
+    MC_CUDA(h, cudaMemcpyAsync(p->pin_codes_out, p->dev_codes_out, (size_t)rows * keep * 8, cudaMemcpyDeviceToHost, stream));
+    return MC_OK;
+  };
+  MC_TRY(run_or_replay(p, std::make_tuple(4, T_max, len, cut, n, keep), stream, body));
+  MC_CUDA(h, cudaStreamSynchronize(stream));
+  memcpy(codes_out, p->pin_codes_out, (size_t)rows * keep * 8);
+  for (int j = 0; j < n; ++j) { p->acur[slots[j]] ^= 1; p->audio_len[slots[j]] = p->pin_table[4 * j + 3]; }
+  return MC_OK;
+}
+
+int mc_pool_push_codes_ragged(mc_pool* p, const int32_t* slots, int32_t n, const int64_t* codes, int32_t len, int32_t keep_samples,
+                              float* wav_out, int32_t* samples_out, mc_stream_t stream_) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  int common = 0;
+  MC_TRY(pool_check_slots(p, slots, n, p->code_len, &common, "mc_pool_push_codes_ragged", false));
+  if (!codes || !wav_out || !samples_out || len < 1) return h->fail(MC_ERR_ARG, "mc_pool_push_codes_ragged: bad arguments");
+  if (len > p->cap_frames) return h->fail(MC_ERR_ARG, "mc_pool_push_codes_ragged: %d frames exceed the capacity %d", len, p->cap_frames);
+  int hop = 1;
+  for (int i = 0; i < h->spec.n_convs; ++i) hop *= h->spec.conv_strides[i];
+  if (keep_samples < 1 || keep_samples > p->cap_frames * hop)
+    return h->fail(MC_ERR_ARG, "mc_pool_push_codes_ragged: keep_samples %d outside 1..%d", keep_samples, p->cap_frames * hop);
+  const int C = p->C, rows = n * C;
+  if (common >= 0) {
+    int got = 0;
+    MC_TRY(mc_pool_push_codes(p, slots, n, codes, len, keep_samples, wav_out, &got, stream_));
+    for (int r = rows - 1; r >= 1 && got < keep_samples; --r)    // rows of `got` samples -> rows of keep_samples, back to front
+      memmove(wav_out + (size_t)r * keep_samples, wav_out + (size_t)r * got, (size_t)got * 4);
+    for (int r = 0; r < rows && got < keep_samples; ++r)
+      memset(wav_out + (size_t)r * keep_samples + got, 0, (size_t)(keep_samples - got) * 4);
+    for (int j = 0; j < n; ++j) samples_out[j] = got;
+    return MC_OK;
+  }
+  MC_TRY(pool_ragged_causal(p, "mc_pool_push_codes_ragged"));
+  MC_CUDA(h, cudaEventRecord(p->order_ev, (cudaStream_t)stream_));
+  MC_CUDA(h, cudaStreamWaitEvent(p->own, p->order_ev, 0));
+  cudaStream_t stream = p->own;
+  const int cap = p->cap_frames;
+  const int F_max = pool_fill_ragged_table(p, slots, n, len, p->ctx_frames, p->code_len, p->ccur);
+  int cut = 0, dec_keep = 0;
+  ragged_decode_cut(p, n, F_max, hop, keep_samples, &cut, &dec_keep);
+  for (int r = 0; r < rows; ++r) memcpy(p->pin_codes_in + (size_t)r * cap, codes + (size_t)r * len, (size_t)len * 8);
+  auto body = [&]() -> int {
+    MC_CUDA(h, cudaMemcpyAsync(p->dev_table, p->pin_table, (size_t)n * 16, cudaMemcpyHostToDevice, stream));
+    MC_CUDA(h, cudaMemcpy2DAsync(p->dev_codes_in, (size_t)cap * 8, p->pin_codes_in, (size_t)cap * 8, (size_t)len * 8, rows, cudaMemcpyHostToDevice, stream));
+    pool_roll_ragged_kernel<long long><<<dim3((F_max + 255) / 256, rows), 256, 0, stream>>>(
+        p->dev_table, C, cap, len, reinterpret_cast<long long*>(p->codes[0]), reinterpret_cast<long long*>(p->codes[1]),
+        reinterpret_cast<const long long*>(p->dev_codes_in), reinterpret_cast<long long*>(p->batch_codes), F_max, F_max);
+    MC_LAUNCH_CHECK(h, "pool_roll_ragged_kernel");
+    MC_TRY(decode_impl(h, p->batch_codes, nullptr, rows, F_max, dec_keep, p->dev_wav_out, stream));
+    pool_gather_samples_ragged_kernel<<<dim3((keep_samples + 255) / 256, rows), 256, 0, stream>>>(
+        p->dev_wav_out, dec_keep, p->dev_table, C, F_max * hop, hop, keep_samples, p->pin_wav_out);   // straight into pinned host memory
+    MC_LAUNCH_CHECK(h, "pool_gather_samples_ragged_kernel");
+    return MC_OK;
+  };
+  MC_TRY(run_or_replay(p, std::make_tuple(5, F_max, len, cut, n, keep_samples), stream, body));
+  MC_CUDA(h, cudaStreamSynchronize(stream));
+  memcpy(wav_out, p->pin_wav_out, (size_t)rows * keep_samples * 4);
+  for (int j = 0; j < n; ++j) {
+    samples_out[j] = std::min(keep_samples, p->pin_table[4 * j + 3] * hop);
+    p->ccur[slots[j]] ^= 1;
+    p->code_len[slots[j]] = p->pin_table[4 * j + 3];
+  }
+  return MC_OK;
+}
+
+int mc_pool_push_codes_emit_ragged(mc_pool* p, const int32_t* slots, int32_t n, const int64_t* codes, int32_t len, float* out,
+                                   int32_t* had_prev, mc_stream_t stream_) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  int common = 0;
+  MC_TRY(pool_check_slots(p, slots, n, p->code_len, &common, "mc_pool_push_codes_emit_ragged", false));
+  if (!codes || !out || !had_prev || len < 1) return h->fail(MC_ERR_ARG, "mc_pool_push_codes_emit_ragged: bad arguments");
+  if (len > p->cap_frames)
+    return h->fail(MC_ERR_ARG, "mc_pool_push_codes_emit_ragged: %d frames exceed the capacity %d", len, p->cap_frames);
+  if (p->C != 1) return h->fail(MC_ERR_ARG, "mc_pool_push_codes_emit_ragged: the emit chain is mono (pad_or_trim rejects [C,T])");
+  if (p->emit_chunk <= 0) return h->fail(MC_ERR_STATE, "mc_pool_push_codes_emit_ragged: call mc_pool_set_emit first");
+  int hop = 1;
+  for (int i = 0; i < h->spec.n_convs; ++i) hop *= h->spec.conv_strides[i];
+  const int chunk = p->emit_chunk, fade = p->emit_fade, cap = p->cap_frames;
+  if (len * hop != chunk)
+    return h->fail(MC_ERR_ARG, "mc_pool_push_codes_emit_ragged: %d codes decode to %d samples, chunk is %d", len, len * hop, chunk);
+  // the stream's rules (realtime_agent_v2.py:566-568) for every slot, before any work or state change
+  for (int j = 0; j < n; ++j) {
+    const int keep = std::min(std::min(p->code_len[slots[j]] + len, std::max(len, p->ctx_frames)) * hop, chunk + fade);
+    if (p->emit_has_prev[slots[j]] && keep != chunk + fade)
+      return h->fail(MC_ERR_STATE, "mc_pool_push_codes_emit_ragged: slot %d: only %d decoded samples for chunk %d + fade %d", slots[j],
+                     keep, chunk, fade);
+    if (!p->emit_has_prev[slots[j]] && keep != chunk)
+      return h->fail(MC_ERR_STATE, "mc_pool_push_codes_emit_ragged: slot %d: the first emitted chunk needs an empty code context (reset first)",
+                     slots[j]);
+  }
+  if (common >= 0) {   // equal lengths: equal keeps, so the rules above leave one shared had_prev
+    int hp = 0;
+    MC_TRY(mc_pool_push_codes_emit(p, slots, n, codes, len, out, &hp, stream_));
+    for (int j = 0; j < n; ++j) had_prev[j] = hp;
+    return MC_OK;
+  }
+  MC_TRY(pool_ragged_causal(p, "mc_pool_push_codes_emit_ragged"));
+  MC_CUDA(h, cudaEventRecord(p->order_ev, (cudaStream_t)stream_));
+  MC_CUDA(h, cudaStreamWaitEvent(p->own, p->order_ev, 0));
+  cudaStream_t stream = p->own;
+  const int block = 2 * chunk + fade;
+  const int F_max = pool_fill_ragged_table(p, slots, n, len, p->ctx_frames, p->code_len, p->ccur);
+  int cut = 0, dec_keep = 0;
+  ragged_decode_cut(p, n, F_max, hop, chunk + fade, &cut, &dec_keep);
+  for (int j = 0; j < n; ++j) memcpy(p->pin_codes_in + (size_t)j * cap, codes + (size_t)j * len, (size_t)len * 8);
+  auto body = [&]() -> int {
+    MC_CUDA(h, cudaMemcpyAsync(p->dev_table, p->pin_table, (size_t)n * 16, cudaMemcpyHostToDevice, stream));
+    MC_CUDA(h, cudaMemcpy2DAsync(p->dev_codes_in, (size_t)cap * 8, p->pin_codes_in, (size_t)cap * 8, (size_t)len * 8, n, cudaMemcpyHostToDevice, stream));
+    pool_roll_ragged_kernel<long long><<<dim3((F_max + 255) / 256, n), 256, 0, stream>>>(
+        p->dev_table, 1, cap, len, reinterpret_cast<long long*>(p->codes[0]), reinterpret_cast<long long*>(p->codes[1]),
+        reinterpret_cast<const long long*>(p->dev_codes_in), reinterpret_cast<long long*>(p->batch_codes), F_max, F_max);
+    MC_LAUNCH_CHECK(h, "pool_roll_ragged_kernel");
+    MC_TRY(decode_impl(h, p->batch_codes, nullptr, n, F_max, dec_keep, p->dev_wav_out, stream));
+    mc_launch(h, emit_chunk_pool_ragged_kernel, dim3(n), dim3(POST_THREADS), 0, stream, (const float*)p->dev_wav_out, (long long)dec_keep,
+              (const int*)p->dev_table, F_max * hop, hop, chunk, fade, p->emit_target_rms, p->emit_silence_thr,
+              (const float*)p->emit_fade_in, p->emit_prev_tails, p->pin_emit);   // the blocks land in pinned host memory directly
+    MC_LAUNCH_CHECK(h, "emit_chunk_pool_ragged_kernel");
+    return MC_OK;
+  };
+  MC_TRY(run_or_replay(p, std::make_tuple(6, F_max, len, cut, n, 0), stream, body));
+  MC_CUDA(h, cudaStreamSynchronize(stream));
+  memcpy(out, p->pin_emit, (size_t)n * block * 4);
+  for (int j = 0; j < n; ++j) {
+    had_prev[j] = p->emit_has_prev[slots[j]];
+    p->ccur[slots[j]] ^= 1;
+    p->code_len[slots[j]] = p->pin_table[4 * j + 3];
+    p->emit_has_prev[slots[j]] = 1;
+  }
+  return MC_OK;
+}
+
+int mc_pool_graph_count(mc_pool* p, int32_t* keys, int32_t* captured) {
+  if (!p) return MC_ERR_ARG;
+  int c = 0;
+  for (const auto& kv : p->graphs) c += kv.second.exec != nullptr;
+  if (keys) *keys = (int32_t)p->graphs.size();
+  if (captured) *captured = c;
   return MC_OK;
 }
 

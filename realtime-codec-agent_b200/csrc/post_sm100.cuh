@@ -246,4 +246,84 @@ pool_roll_kernel(const int* __restrict__ table, int C, int cap, int old_len, int
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Ragged session-pool batches (mc_pool_push_*_ragged): the items' contexts differ in length.  The encoder and decoder
+// are causal for window_right == 0, so every item's window starts at row 0 of the batch and reads zeros (audio) or
+// code 0 (codes) past its own end; its frames are then bit-identical to its lone pass (DESIGN.md §4 "Warm-up prefixes").
+//   rtable[4j .. 4j+3] = {slot, context buffer, old_len, new_len} of batch item j
+// ---------------------------------------------------------------------------------------------
+// pool_roll_kernel per item, plus the zero fill: batch row j*C + c = the item's new_len values, then zeros up to `width`
+// (T_max samples or F_max frames).
+template <typename T>
+__global__ void __launch_bounds__(256)
+pool_roll_ragged_kernel(const int* __restrict__ rtable, int C, int cap, int n_new, T* __restrict__ ctx0, T* __restrict__ ctx1,
+                        const T* __restrict__ staged /*[n*C, cap]*/, T* __restrict__ batch, int batch_ld, int width) {
+  const int jc = blockIdx.y;
+  const int j = jc / C, c = jc - j * C;
+  const int slot = rtable[4 * j], par = rtable[4 * j + 1], old_len = rtable[4 * j + 2], new_len = rtable[4 * j + 3];
+  const int keep_old = new_len - n_new;
+  const T* src = (par ? ctx1 : ctx0) + (static_cast<long long>(slot) * C + c) * cap;
+  T* dst = (par ? ctx0 : ctx1) + (static_cast<long long>(slot) * C + c) * cap;
+  const T* st = staged + static_cast<long long>(jc) * cap;
+  T* bt = batch + static_cast<long long>(jc) * batch_ld;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < width; i += gridDim.x * blockDim.x) {
+    if (i < new_len) {
+      const T v = i < keep_old ? src[old_len - keep_old + i] : st[i - keep_old];
+      dst[i] = v;
+      bt[i] = v;
+    } else {
+      bt[i] = T(0);
+    }
+  }
+}
+
+// Encode: z [n*C, rows, dq] holds the last `rows` frames of every F_max-frame window; item j keeps its own last `keep`
+// frames, rows [F_j - keep, F_j) of its window with F_j = ceil(new_len_j / hop).  out [n*C, keep, dq], dense for the VQ.
+__global__ void __launch_bounds__(256)
+pool_gather_rows_ragged_kernel(const float* __restrict__ z, const int* __restrict__ rtable, int C, int rows, int F_max, int keep,
+                               int dq, int hop, float* __restrict__ out) {
+  const int jc = blockIdx.y, j = jc / C;
+  const int F_j = (rtable[4 * j + 3] + hop - 1) / hop;
+  const int r0 = rows - (F_max - F_j) - keep;
+  const float* src = z + (static_cast<long long>(jc) * rows + r0) * dq;
+  float* dst = out + static_cast<long long>(jc) * keep * dq;
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < keep * dq; e += gridDim.x * blockDim.x) dst[e] = src[e];
+}
+
+// Decode: wav [n*C, ld] holds the last ld samples of every F_max*hop-sample window; item j keeps
+// k_j = min(keep, new_len_j*hop) samples ending at its own end.  out [n*C, keep] (pinned host memory): the k_j samples at
+// the row start, zeros after them.
+__global__ void __launch_bounds__(256)
+pool_gather_samples_ragged_kernel(const float* __restrict__ wav, long long ld, const int* __restrict__ rtable, int C, int total_max,
+                                  int hop, int keep, float* __restrict__ out) {
+  const int jc = blockIdx.y, j = jc / C;
+  const int total_j = rtable[4 * j + 3] * hop;
+  const int k = min(keep, total_j);
+  const long long off = ld - (total_max - total_j) - k;
+  const float* w = wav + jc * ld + off;
+  float* o = out + static_cast<long long>(jc) * keep;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < keep; i += gridDim.x * blockDim.x) o[i] = i < k ? w[i] : 0.0f;
+}
+
+// emit_chunk_pool_kernel for a ragged batch: wav as for pool_gather_samples_ragged_kernel.  Item j's decoded samples are
+// the last min(new_len_j*hop, chunk + L) of its window: chunk + L for a continuing chunk, chunk for a first one (the host
+// checks that these agree with each slot's state), so has_prev and n_have are per item.
+__global__ void __launch_bounds__(POST_THREADS)
+emit_chunk_pool_ragged_kernel(const float* __restrict__ wav, long long ld, const int* __restrict__ rtable, int total_max, int hop,
+                              int chunk, int L, float target_rms, float silence_thr, const float* __restrict__ fade_in,
+                              float* __restrict__ prev_tails, float* __restrict__ out) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ double scratch[POST_THREADS / 32 + 1];
+  const int j = blockIdx.x;
+  const long long slot = rtable[4 * j];
+  const int total_j = rtable[4 * j + 3] * hop;
+  const int keep = min(total_j, chunk + L);
+  const long long off = ld - (total_max - total_j) - keep;
+  // keep == chunk + L <=> a continuing chunk: mc_pool_push_codes_emit_ragged rejects any slot whose keep disagrees with
+  // its state (first chunk: keep == chunk), and mc_pool_set_emit enforces L >= 1, so the two cases never coincide
+  emit_chunk_body(wav + j * ld + off, keep, chunk, L, keep == chunk + L ? 1 : 0, target_rms, silence_thr, fade_in,
+                  prev_tails + slot * L, out + static_cast<long long>(j) * (2 * chunk + L), scratch);
+}
+
 }  // namespace mc

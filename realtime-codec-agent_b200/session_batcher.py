@@ -10,7 +10,9 @@ same time go through the engine as ONE ``B = n * channels`` launch.
 ``SessionBatcher`` keeps, per session, exactly the host-side state of ``AudioTokenizer`` (context length, code
 string context, the ``[-0:]`` / hanging-code quirks of audio_tokenizer.py:99-101,144,161-168), so every session's
 outputs are what its own ``AudioTokenizer`` would have returned.  Sessions whose contexts differ in length (a stream
-that has just started next to one in steady state) are grouped by length: one launch per group.
+that has just started next to one in steady state) are grouped by length: one launch per group.  With
+``ragged=True`` they share one launch (``mc_pool_push_*_ragged``): each window starts at row 0 of the batch and reads
+zeros past its own end, which the causal codec never looks at.
 
 ``SessionBatcher.emit_output_chunks`` is ``OutputChunkEmitter.emit`` for many agents at once: decoder, ``pad_or_trim``,
 ``normalize_audio_rms`` and ``smooth_join`` of every session of a group run as ONE engine call (``mc_pool_push_codes_emit``,
@@ -105,6 +107,51 @@ class SessionPool:
             nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_push_codes_emit")
         return out, bool(had.value)
 
+    def push_audio_ragged(self, slots, chunks: np.ndarray, keep_frames: int) -> np.ndarray:
+        """push_audio for sessions whose contexts may differ in length: chunks float32 [n, C, len] -> int64 codes
+        [n, C, keep_frames], each session's own last keep_frames frames (1 <= keep_frames <= ceil(len / hop))."""
+        slots = np.ascontiguousarray(slots, dtype=np.int32)
+        chunks = np.ascontiguousarray(chunks, dtype=np.float32).reshape(len(slots), self.channels, -1)
+        out = np.empty((len(slots), self.channels, keep_frames), dtype=np.int64)
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_push_audio_ragged(self._p, slots.ctypes.data, len(slots), chunks.ctypes.data, chunks.shape[2],
+                                                         keep_frames, out.ctypes.data, self.gen._stream())
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_push_audio_ragged")
+        return out
+
+    def push_codes_ragged(self, slots, codes: np.ndarray, keep_samples: int) -> Tuple[np.ndarray, np.ndarray]:
+        """push_codes for sessions whose contexts may differ in length: codes int64 [n, C, len] -> (float32 wav
+        [n, C, keep_samples], int32 samples [n]); session j's samples fill the first samples[j] of its row."""
+        slots = np.ascontiguousarray(slots, dtype=np.int32)
+        codes = np.ascontiguousarray(codes, dtype=np.int64).reshape(len(slots), self.channels, -1)
+        out = np.empty((len(slots), self.channels, keep_samples), dtype=np.float32)
+        got = np.zeros(len(slots), dtype=np.int32)
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_push_codes_ragged(self._p, slots.ctypes.data, len(slots), codes.ctypes.data, codes.shape[2],
+                                                         keep_samples, out.ctypes.data, got.ctypes.data, self.gen._stream())
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_push_codes_ragged")
+        return out, got
+
+    def push_codes_emit_ragged(self, slots, codes: np.ndarray) -> Tuple[np.ndarray, np.ndarray]:
+        """push_codes_emit for sessions whose contexts may differ in length, first chunks mixed with continuing ones:
+        codes int64 [n, len] -> (float32 [n, 2*chunk + fade], bool had_prev [n])."""
+        slots = np.ascontiguousarray(slots, dtype=np.int32)
+        codes = np.ascontiguousarray(codes, dtype=np.int64).reshape(len(slots), -1)
+        out = np.empty((len(slots), getattr(self, "_emit_floats", 0)), dtype=np.float32)
+        had = np.zeros(len(slots), dtype=np.int32)
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_push_codes_emit_ragged(self._p, slots.ctypes.data, len(slots), codes.ctypes.data,
+                                                              codes.shape[1], out.ctypes.data, had.ctypes.data, self.gen._stream())
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_push_codes_emit_ragged")
+        return out, had.astype(bool)
+
+    def graph_count(self) -> Tuple[int, int]:
+        """(distinct graph keys seen, graphs captured) over every push of this pool."""
+        k, c = C.c_int32(), C.c_int32()
+        with self.gen._serial():
+            self.gen._lib.mc_pool_graph_count(self._p, C.byref(k), C.byref(c))
+        return k.value, c.value
+
     def __del__(self):
         try:
             if getattr(self, "_p", None) and self.gen._handle:
@@ -126,10 +173,14 @@ class SessionBatcher:
     """Batched ``tokenize_audio`` / ``detokenize_audio`` over many independent sessions of one engine."""
 
     def __init__(self, codec_model, num_channels: int = 1, context_secs: float = 2.0, max_sessions: int = 8,
-                 unicode_offset: int = UNICODE_OFFSET_LARGE):
+                 unicode_offset: int = UNICODE_OFFSET_LARGE, ragged: bool = False):
+        """ragged=True: sessions whose contexts differ in length go through one engine call per kind and tick (split only by
+        chunk length, and by decode length and preroll) instead of one call per context length.  Off by default: with the
+        default split-K kernels a mixed batch has another row count than today's groups, so near-tie codes may change."""
         if not getattr(codec_model, "is_b200_native", False):
             raise RuntimeError("SessionBatcher needs the B200 engine (B200Generator); there is no fallback")
         self.gen = codec_model
+        self.ragged = ragged
         self.num_channels, self.context_secs, self.unicode_offset = num_channels, context_secs, unicode_offset
         self.sampling_rate = codec_model.sample_rate
         self.framerate = self.sampling_rate / codec_model.hop
@@ -185,13 +236,16 @@ class SessionBatcher:
                 if not 0 < x.shape[1] <= self.pool.cap_samples:
                     raise ValueError(f"session {sid}: chunks must hold 1..{self.pool.cap_samples} samples")
                 prepped[sid] = x
-                groups.setdefault((self._sessions[sid].audio_len, x.shape[1]), []).append(sid)
+                # ragged: one call per chunk length; the [-0:] case keeps every frame of each window, so it stays grouped
+                ragged = self.ragged and self._n_chars(x.shape[1]) > 0
+                groups.setdefault((-1 if ragged else self._sessions[sid].audio_len, x.shape[1]), []).append(sid)
             out: Dict[int, str] = {}
-            for (_, n_new), sids in groups.items():
-                n_chars = int(n_new / self.sampling_rate * self.framerate * C_)
+            for (ctx_len, n_new), sids in groups.items():
+                n_chars = self._n_chars(n_new)
                 frames_needed = -(-n_chars // C_) if n_chars > 0 else 0                  # 0 -> all frames ([-0:])
                 slots = [self._sessions[s].slot for s in sids]
-                codes = self.pool.push_audio(slots, np.stack([prepped[s] for s in sids]), frames_needed)   # [n,C,k]
+                push = self.pool.push_audio_ragged if ctx_len < 0 else self.pool.push_audio
+                codes = push(slots, np.stack([prepped[s] for s in sids]), frames_needed)   # [n,C,k]
                 for j, sid in enumerate(sids):
                     st = self._sessions[sid]
                     st.audio_len = min(st.audio_len + n_new, max(n_new, self.context_samples))
@@ -199,6 +253,9 @@ class SessionBatcher:
                     text = codes_to_chars(frame_major, self.codebook_size, unicode_offset=self.unicode_offset)
                     out[sid] = text[-n_chars:]
             return out
+
+    def _n_chars(self, n_new: int) -> int:
+        return int(n_new / self.sampling_rate * self.framerate * self.num_channels)
 
     # ---- decode
     def detokenize_audio(self, strings: Dict[int, str], preroll_samples: int = 0):
@@ -226,12 +283,17 @@ class SessionBatcher:
                 st = self._sessions[sid]
                 st.detok_context = (st.detok_context + s)[-max(len(s), self.context_frames):]
                 wants[sid] = int(len(s) / (self.framerate * C_) * self.sampling_rate) + preroll_samples
-                ctx_frames_before = self.pool.context_len(st.slot)[1]
+                ctx_frames_before = -1 if self.ragged else self.pool.context_len(st.slot)[1]
                 groups.setdefault((ctx_frames_before, len(s) // C_, wants[sid]), []).append(sid)
             out = {}
-            for (_, _, want), sids in groups.items():
+            for (ctx_len, _, want), sids in groups.items():
                 slots = [self._sessions[s].slot for s in sids]
-                wav = self.pool.push_codes(slots, np.stack([new_codes[s] for s in sids]), want)   # [n,C,k]
+                codes = np.stack([new_codes[s] for s in sids])
+                if ctx_len < 0:       # no window holds more than cap_frames * hop samples: the clamp changes no session's samples
+                    wav, got = self.pool.push_codes_ragged(slots, codes, min(want, self.pool.cap_frames * self.gen.hop))
+                    wav = [wav[j][..., :got[j]] for j in range(len(sids))]
+                else:
+                    wav = self.pool.push_codes(slots, codes, want)   # [n,C,k]
                 for j, sid in enumerate(sids):
                     w = wav[j]
                     preroll_left = max(0, preroll_samples - want + w.shape[-1])
@@ -263,7 +325,7 @@ class SessionBatcher:
     def emit_output_chunks(self, strings: Dict[int, str]) -> Dict[int, np.ndarray]:
         """{session: output code string of one chunk} -> {session: float32 [chunk]}, each exactly what that session's own
         ``OutputChunkEmitter.emit`` returns; the code contexts advance as in ``detokenize_audio``.  Sessions are grouped by
-        code-context length, one engine call per group."""
+        code-context length, one engine call per group (ragged: one call for all of them)."""
         with self._lock:
             if self._emit is None:
                 raise ValueError("call arm_emit first")
@@ -279,20 +341,24 @@ class SessionBatcher:
                 if not st.history and st.detok_context:
                     raise ValueError(f"session {sid}: the first emitted chunk needs an empty code context (reset_context first)")
                 new_codes[sid] = chars_to_codes(s, 1, self.codebook_size, unicode_offset=self.unicode_offset)[0]
-                ctx_frames_before = self.pool.context_len(st.slot)[1]
-                groups.setdefault((ctx_frames_before, bool(st.history)), []).append(sid)
+                key = (-1, None) if self.ragged else (self.pool.context_len(st.slot)[1], bool(st.history))
+                groups.setdefault(key, []).append(sid)
             for sid, s in strings.items():
                 st = self._sessions[sid]
                 st.detok_context = (st.detok_context + s)[-max(len(s), self.context_frames):]
             out = {}
-            for (_, has_prev), sids in groups.items():
-                blocks, had_prev = self.pool.push_codes_emit([self._sessions[s].slot for s in sids],
-                                                             np.stack([new_codes[s] for s in sids]))
-                if had_prev != has_prev:
-                    raise RuntimeError("emit chain state diverged from audio_history_ch1")
+            for (ctx_len, has_prev), sids in groups.items():
+                slots, codes = [self._sessions[s].slot for s in sids], np.stack([new_codes[s] for s in sids])
+                if ctx_len < 0:
+                    blocks, had = self.pool.push_codes_emit_ragged(slots, codes)
+                else:
+                    blocks, had_prev = self.pool.push_codes_emit(slots, codes)
+                    had = [had_prev] * len(sids)
                 for j, sid in enumerate(sids):                   # OutputChunkEmitter._emit_native, session by session
                     block, hist = blocks[j], self._sessions[sid].history
-                    if had_prev:
+                    if bool(had[j]) != bool(hist):
+                        raise RuntimeError("emit chain state diverged from audio_history_ch1")
+                    if had[j]:
                         hist[-1] = np.concatenate((hist[-1][:chunk - L], block[chunk:chunk + L]))
                     hist.append(block[chunk + L:].copy())
                     out[sid] = block[:chunk].copy()
