@@ -563,6 +563,22 @@ int stem_prefix_frames(const mc_spec& s) {
   return (int)dirty;
 }
 
+// Frames a decode cut from a longer window needs before its first kept sample.  Transposed conv i (stride ds[i]) reads
+// input steps t−1 and t, so the zero left pad of a cut window spoils its first ds[i] outputs, and the spoiled prefix
+// grows through the stack to L = Σ_i hop / Π_{j<i} ds[j] samples (404 for strides (4, 4, 4, 5)).  The margin is
+// ceil(L / hop): 2 frames for the default strides, more when a late encoder stride is small (3 for (4, 4, 5, 1)).
+int tconv_margin_frames(const mc_spec& s) {
+  const int n = s.n_convs;
+  int hop = 1;
+  for (int i = 0; i < n; ++i) hop *= s.conv_strides[i];
+  long long look_back = 0, step = hop;   // step: samples per input position of decoder conv i
+  for (int i = 0; i < n; ++i) {
+    look_back += step;
+    step /= s.conv_strides[n - 1 - i];
+  }
+  return (int)((look_back + hop - 1) / hop);
+}
+
 // A ragged session-pool batch (mc_pool_push_audio_ragged): encode_impl's `keep` rows of every window run through the
 // stack, then each item's own last `keep` frames (rtable: pool_roll_ragged_kernel's table) are gathered for the VQ.
 struct RaggedKeep {
@@ -688,9 +704,8 @@ int decode_impl(mc_handle* h, const int64_t* codes, const float* z_q, int B, int
     ds[i] = s.conv_strides[n - 1 - i];
     dch[i + 1] = (n - 2 - i >= 0) ? s.conv_channels[n - 2 - i] : 1;
   }
-  // Frames whose samples are kept, plus two more: the causal transposed convs look one step back at
-  // every rate, so a window cut at frame f0 has wrong samples only in its first 404 (< 2 frames).
-  const int Rk = (keep >= total) ? F : std::min(F, (keep + hop - 1) / hop + 2);
+  // Frames whose samples are kept, plus the margin the causal transposed convs look back over (tconv_margin_frames).
+  const int Rk = (keep >= total) ? F : std::min(F, (keep + hop - 1) / hop + tconv_margin_frames(s));
   Tin[0] = Rk;
   for (int i = 1; i < n; ++i) Tin[i] = Tin[i - 1] * ds[i - 1];
 
@@ -759,6 +774,9 @@ int decode_impl(mc_handle* h, const int64_t* codes, const float* z_q, int B, int
     if (ds[i] > 8 || dch[i] % 8 != 0) return h->fail(MC_ERR_ARG, "last tconv: stride %d / channels %d unsupported", ds[i], dch[i]);
     const long long items = (long long)B * Tin[i];
     const size_t smem = (size_t)dch[i] * 2 * ds[i] * 4;
+    // the weight table outgrows the default 48 KB from Cin * stride > 6144 on (e.g. 1024 channels at stride 8); the
+    // attribute is per function, so it is raised to the largest table a spec can ask for (2048 channels, stride 8)
+    if (smem > 48 * 1024) MC_TRY(mc_allow_smem(h, tconv_last_kernel<8>, 2048 * 2 * 8 * 4));
     McProfScope prof(h, 3, 4.0 * B * Tin[i] * dch[i] * ds[i], (double)B * Tin[i] * dch[i] * 2.0 + (double)B * keep * 4.0, stream);
     mc_launch(h, tconv_last_kernel<8>, dim3(ew_grid(h, items, threads)), dim3(threads), smem, stream,
               reinterpret_cast<const bf16*>(base + tb_off[i]), B, Tin[i], dch[i], ds[i],
@@ -814,6 +832,38 @@ std::vector<std::string> required_tensors(const mc_spec& s) {
   return v;
 }
 
+// The specs the kernels are built for (the same rules as MagiCodecSpec.validate()); empty if `s` is one of them.
+std::string spec_refusal(const mc_spec& s) {
+  char msg[160];
+  const int n = s.n_convs;
+  if (n < 2 || n > MC_MAX_CONVS) return "need 2 .. " + std::to_string(MC_MAX_CONVS) + " convs";
+  if (s.n_heads < 1 || s.d_model % 64 != 0 || s.d_model / s.n_heads != 64 || s.d_model % s.n_heads != 0 ||
+      s.ffn_dim < 64 || s.ffn_dim % 64 != 0 || s.codebook_dim != 16 || s.codebook_size < 256 || s.codebook_size % 256 != 0 ||
+      s.conv_channels[n - 1] != s.d_model || s.enc_layers < 0 || s.dec_layers < 0)
+    return "need head_dim 64, d/ffn multiples of 64, codebook_dim 16, codebook_size a multiple of 256";
+  if (s.window_left < 0 || s.window_left > 96 || s.window_right < 0 || s.window_right > 32)
+    return "attention window (" + std::to_string(s.window_left) + ", " + std::to_string(s.window_right) +
+           ") too wide: window_left <= 96, window_right <= 32";
+  for (int i = 0; i < n; ++i)
+    if (s.conv_strides[i] < 1 || s.conv_channels[i] < 1) return "conv strides and channels must be positive";
+  const int s0 = s.conv_strides[0], c0 = s.conv_channels[0];
+  if ((s0 != 4 && s0 != 8) || c0 % 8 != 0 || 256 % (c0 / 8) != 0) {
+    snprintf(msg, sizeof msg, "conv0: stride %d / channels %d unsupported (stride 4 or 8, 8 * 2^k channels up to 2048)", s0, c0);
+    return msg;
+  }
+  for (int i = 1; i < n; ++i)
+    if (s.conv_strides[i] * s.conv_channels[i - 1] % 64 != 0) {
+      snprintf(msg, sizeof msg, "conv %d: stride * Cin = %d * %d is not a multiple of 64", i, s.conv_strides[i], s.conv_channels[i - 1]);
+      return msg;
+    }
+  for (int i = 1; i + 1 < n; ++i)   // transposed convs 0 .. n-2 read d and conv_channels[n-2] .. [1] as GEMM K blocks
+    if (s.conv_channels[i] % 64 != 0) {
+      snprintf(msg, sizeof msg, "tconv: %d input channels are not a multiple of 64", s.conv_channels[i]);
+      return msg;
+    }
+  return std::string();
+}
+
 }  // namespace
 
 // =============================================================== C ABI
@@ -834,10 +884,9 @@ int mc_create(const mc_spec* spec, int device, mc_handle** out) {
                      "; this library contains sm_100a code only (no fallback)";
     return MC_ERR_ARCH;
   }
-  if (spec->n_convs < 2 || spec->n_convs > MC_MAX_CONVS || spec->d_model % 64 != 0 || spec->d_model / spec->n_heads != 64 ||
-      spec->ffn_dim % 64 != 0 || spec->codebook_dim != 16 || spec->codebook_size % 256 != 0 ||
-      spec->conv_channels[spec->n_convs - 1] != spec->d_model) {
-    g_create_error = "mc_create: unsupported spec (need head_dim 64, d/ffn multiples of 64, codebook_dim 16)";
+  const std::string refusal = spec_refusal(*spec);
+  if (!refusal.empty()) {
+    g_create_error = "mc_create: unsupported spec: " + refusal;
     return MC_ERR_ARG;
   }
   e = cudaSetDevice(device);
@@ -1613,15 +1662,17 @@ int pool_fill_ragged_table(mc_pool* p, const int32_t* slots, int n, int len, int
 int ragged_cut(int rows, int F) { return std::min(F, (rows + 15) / 16 * 16); }
 
 // Decoder rows of a ragged decode whose items keep keep_j = min(keep, F_j * hop) samples each (the earliest kept sample
-// over the batch, plus the two frames the transposed convs look back), and the `keep` decode_impl takes for that cut.
+// over the batch, plus the frames the transposed convs look back: tconv_margin_frames), and the `keep` decode_impl takes
+// for that cut.
 void ragged_decode_cut(const mc_pool* p, int n, int F_max, int hop, int keep, int* rows, int* dec_keep) {
   int need = 0;
   for (int j = 0; j < n; ++j) {
     const int total_j = p->pin_table[4 * j + 3] * hop;
     need = std::max(need, (F_max * hop - total_j) + std::min(keep, total_j));
   }
-  *rows = ragged_cut((need + hop - 1) / hop + 2, F_max);
-  *dec_keep = *rows >= F_max ? F_max * hop : (*rows - 2) * hop;
+  const int margin = tconv_margin_frames(p->h->spec);
+  *rows = ragged_cut((need + hop - 1) / hop + margin, F_max);
+  *dec_keep = *rows >= F_max ? F_max * hop : (*rows - margin) * hop;
 }
 }  // namespace
 

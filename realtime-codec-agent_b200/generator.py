@@ -118,6 +118,23 @@ def pack_weights(spec: MagiCodecSpec, w: Dict[str, torch.Tensor], max_positions:
     return {k: v.contiguous() for k, v in p.items()}
 
 
+def mc_spec_struct(spec: MagiCodecSpec, max_positions: int) -> nat.McSpec:
+    """The C ABI's mc_spec for `spec` (not validated: mc_create applies the same rules as spec.validate())."""
+    cs = nat.McSpec()
+    cs.sample_rate, cs.n_convs = spec.sample_rate, len(spec.conv_strides)
+    for i, c in enumerate(tuple(spec.conv_channels) + (spec.d_model,)):
+        cs.conv_channels[i] = c
+    for i, s in enumerate(spec.conv_strides):
+        cs.conv_strides[i] = s
+    cs.d_model, cs.n_heads, cs.ffn_dim = spec.d_model, spec.n_heads, spec.ffn_dim
+    cs.enc_layers, cs.dec_layers = spec.enc_layers, spec.dec_layers
+    cs.window_left, cs.window_right = spec.window_left, spec.window_right
+    cs.norm_eps = spec.norm_eps
+    cs.codebook_size, cs.codebook_dim = spec.codebook_size, spec.codebook_dim
+    cs.max_positions = max_positions
+    return cs
+
+
 # ------------------------------------------------------------------------------- streaming
 class StreamSession:
     """Device-resident rolling context of one AudioTokenizer (mc_stream_* in the C ABI): each push
@@ -302,18 +319,7 @@ class B200Generator:
         self.max_positions = max_positions
         self._lib = nat.load_library()
         self._handle = C.c_void_p()
-        cs = nat.McSpec()
-        cs.sample_rate, cs.n_convs = spec.sample_rate, len(spec.conv_strides)
-        for i, c in enumerate(tuple(spec.conv_channels) + (spec.d_model,)):
-            cs.conv_channels[i] = c
-        for i, s in enumerate(spec.conv_strides):
-            cs.conv_strides[i] = s
-        cs.d_model, cs.n_heads, cs.ffn_dim = spec.d_model, spec.n_heads, spec.ffn_dim
-        cs.enc_layers, cs.dec_layers = spec.enc_layers, spec.dec_layers
-        cs.window_left, cs.window_right = spec.window_left, spec.window_right
-        cs.norm_eps = spec.norm_eps
-        cs.codebook_size, cs.codebook_dim = spec.codebook_size, spec.codebook_dim
-        cs.max_positions = max_positions
+        cs = mc_spec_struct(spec, max_positions)
         rc = self._lib.mc_create(C.byref(cs), self.device.index, C.byref(self._handle))
         nat.check(self._lib, None, rc, "mc_create")
         packed = pack_weights(spec, weights, max_positions)

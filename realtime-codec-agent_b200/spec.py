@@ -81,6 +81,12 @@ class MagiCodecSpec:
         assert self.codebook_size % 256 == 0
         assert 0 <= self.window_left <= 96 and 0 <= self.window_right <= 32
         ch = self.enc_channels
+        s0, c0 = self.conv_strides[0], ch[1]
+        # conv_first_kernel is instantiated for 8 and 16 taps and gives each thread 8 channels of a 256-thread block;
+        # the last transposed conv (Cout = 1) mirrors it and reads 16-byte groups of 8 channels
+        assert s0 in (4, 8), f"conv 0: stride {s0} unsupported (the first conv runs strides 4 and 8)"
+        assert c0 % 8 == 0 and 256 % (c0 // 8) == 0, \
+            f"conv 0: {c0} channels unsupported (need 8 * 2^k channels, at most 2048)"
         for i, s in enumerate(self.conv_strides):
             if i >= 1:
                 # GEMM convs: the K loop walks stride*Cin-wide row blocks in 64-element steps
