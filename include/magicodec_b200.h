@@ -220,6 +220,42 @@ int mc_pool_push_codes_ragged(mc_pool* p, const int32_t* slots, int32_t n, const
 int mc_pool_push_codes_emit_ragged(mc_pool* p, const int32_t* slots, int32_t n, const int64_t* codes, int32_t len, float* out,
                                    int32_t* had_prev, mc_stream_t stream);
 int mc_pool_graph_count(mc_pool* p, int32_t* keys, int32_t* captured);
+/* The last n samples (1 <= n <= the slot's context length) of a slot's audio context -> HOST fp32 [C][n]. */
+int mc_pool_read_audio(mc_pool* p, int32_t slot, float* out_host, int32_t n);
+
+/* ---- live-stream ingest for pooled sessions whose clients send PCM at their own rate and sample format (48 / 44.1 kHz
+ * int16 from WebRTC or a TTS engine): per chunk what AudioTokenizer._prep_audio_for_tokenization does on the host
+ * (audio_tokenizer.py:203-215: int16 / 32768, the mean over channels for a mono codec, librosa.resample), done on the
+ * device inside the push's graph.  Each chunk is resampled on its own with zero edges, as the reference does.
+ * set_resampler: registers the polyphase plan of one input rate (the ResamplePlan of audio_io.resample_plan(sr_in, codec
+ * rate): taps HOST fp32 [n_taps], already scaled by `up` and left-padded; pre_remove = leading outputs dropped).
+ *   sr_in * up == codec rate * down; at most MC_POOL_MAX_RESAMPLERS rates per pool; registering a rate again replaces it.
+ * reserve_pcm: fixes the pinned staging of the raw chunks at max_sessions chunks of max_in_channels x max_in_samples;
+ *   afterwards a larger item fails with MC_ERR_ARG.  Without it the staging is sized at first use and grows when a call
+ *   needs more.
+ * push_pcm / push_pcm_ragged: mc_pool_push_audio / mc_pool_push_audio_ragged (same rules, same results) on the converted
+ *   samples.  items HOST [n]: item j's chunk is planar [channels_in][ld] samples (MC_PCM_S16 or MC_PCM_F32, native byte
+ *   order) at payload + offset_bytes, n_in per channel, at sample_rate (the codec's rate, or a registered one).  Every
+ *   item must resample to `len` samples, ceil(n_in * up / down).  A pool with C > 1 channels needs channels_in == C; a
+ *   mono pool takes 1..MC_POOL_MAX_MIX_CHANNELS channels and mixes them (fp32 mean, np.mean(axis=0) order).  Per item
+ *   the staged samples are bit for bit mc_op_pcm_to_f32 followed by mc_op_resample on the same bytes.  Every check runs
+ *   before any work or state change. */
+#define MC_POOL_MAX_RESAMPLERS 8
+#define MC_POOL_MAX_MIX_CHANNELS 8
+typedef struct mc_pcm_chunk {
+  int32_t format;        /* MC_PCM_S16 or MC_PCM_F32 */
+  int32_t channels_in;
+  int32_t n_in;          /* samples per channel */
+  int32_t sample_rate;
+  int64_t offset_bytes;  /* of channel 0 in payload */
+  int64_t ld;            /* samples from one channel's row to the next */
+} mc_pcm_chunk;
+int mc_pool_set_resampler(mc_pool* p, int32_t sr_in, int32_t up, int32_t down, const float* taps, int32_t n_taps, int64_t pre_remove);
+int mc_pool_reserve_pcm(mc_pool* p, int32_t max_in_samples, int32_t max_in_channels);
+int mc_pool_push_pcm(mc_pool* p, const int32_t* slots, int32_t n, const mc_pcm_chunk* items, const void* payload, int32_t len,
+                     int32_t keep_frames, int64_t* codes_out, int32_t* frames_out, mc_stream_t stream);
+int mc_pool_push_pcm_ragged(mc_pool* p, const int32_t* slots, int32_t n, const mc_pcm_chunk* items, const void* payload, int32_t len,
+                            int32_t keep_frames, int64_t* codes_out, mc_stream_t stream);
 
 /* ids DEVICE int64 [rows, n] (LM token ids; code = id - vocab_start, clamped to the codebook).
  * dist_out DEVICE fp32 [rows] (optional) = mean_j ||E[code_j] - ref||_2, ref DEVICE fp32 [dq] (NULL = 0);

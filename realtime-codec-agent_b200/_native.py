@@ -9,11 +9,18 @@ import ctypes as C
 import os
 from typing import Optional
 
+import numpy as np
 import torch
 
 from .build import LIB_PATH
 
 MC_MAX_CONVS = 8
+MC_POOL_MAX_RESAMPLERS = 8      # input rates one session pool converts on the device
+MC_POOL_MAX_MIX_CHANNELS = 8    # channels a mono pool mixes on the device
+
+#: struct mc_pcm_chunk: one item of mc_pool_push_pcm
+PCM_CHUNK_DTYPE = np.dtype([("format", "<i4"), ("channels_in", "<i4"), ("n_in", "<i4"), ("sample_rate", "<i4"),
+                            ("offset_bytes", "<i8"), ("ld", "<i8")])
 
 
 class McSpec(C.Structure):
@@ -75,6 +82,11 @@ SYMBOLS = {
     "mc_pool_push_codes_ragged": (C.c_int, [_P, _P, _I32, _P, _I32, _I32, _P, _P, _P]),
     "mc_pool_push_codes_emit_ragged": (C.c_int, [_P, _P, _I32, _P, _I32, _P, _P, _P]),
     "mc_pool_graph_count": (C.c_int, [_P, C.POINTER(_I32), C.POINTER(_I32)]),
+    "mc_pool_read_audio": (C.c_int, [_P, _I32, _P, _I32]),
+    "mc_pool_set_resampler": (C.c_int, [_P, _I32, _I32, _I32, _P, _I32, _I64]),
+    "mc_pool_reserve_pcm": (C.c_int, [_P, _I32, _I32]),
+    "mc_pool_push_pcm": (C.c_int, [_P, _P, _I32, _P, _P, _I32, _I32, _P, C.POINTER(_I32), _P]),
+    "mc_pool_push_pcm_ragged": (C.c_int, [_P, _P, _I32, _P, _P, _I32, _I32, _P, _P]),
     "mc_embed_distance": (C.c_int, [_P, _P, _I32, _I32, _I64, _P, _P, _P, _P]),
     "mc_op_gemm": (C.c_int, [_P, _P, _I64, _I32, _P, _P, _I32, _I32, _I32, _I32, _I32, _P, _I64,
                              _I32, _I32, _I64, _I64, _I32, _I32, _I32, _P]),

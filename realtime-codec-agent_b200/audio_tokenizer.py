@@ -432,17 +432,22 @@ class AudioTokenizer:
         return m.decoder(torch.nn.functional.embedding(codes, table)).float()
 
     def _prep_audio_for_tokenization(self, audio: AudioLike) -> np.ndarray:
-        sr, wav = (self.sampling_rate, audio) if isinstance(audio, np.ndarray) else audio
-        if wav.dtype == np.int16:
-            wav = wav.astype("float32") / 32768.0
-        if self.num_channels == 1 and wav.ndim > 1:
-            wav = np.mean(wav, axis=0)                       # librosa.to_mono
-        if sr != self.sampling_rate:
-            wav = _resample(wav, sr, self.sampling_rate)
-        return wav
+        return prep_audio_for_tokenization(audio, self.sampling_rate, self.num_channels)
 
     def _autocast(self):
         return torch.autocast(device_type="cuda", dtype=torch.bfloat16, enabled=self.autocast_bfloat16)
+
+
+def prep_audio_for_tokenization(audio: AudioLike, sampling_rate: int, num_channels: int) -> np.ndarray:
+    """audio_tokenizer.py:203-215: int16 -> float32 / 32768, the mean over channels for a mono codec, the resampler."""
+    sr, wav = (sampling_rate, audio) if isinstance(audio, np.ndarray) else audio
+    if wav.dtype == np.int16:
+        wav = wav.astype("float32") / 32768.0
+    if num_channels == 1 and wav.ndim > 1:
+        wav = np.mean(wav, axis=0)                       # librosa.to_mono
+    if sr != sampling_rate:
+        wav = _resample(wav, sr, sampling_rate)
+    return wav
 
 
 def _resample(wav: np.ndarray, orig_sr: int, target_sr: int) -> np.ndarray:

@@ -1607,6 +1607,14 @@ struct mc_pool {
   float* emit_fade_in = nullptr;   // device [fade]
   float* emit_prev_tails = nullptr;// device [max_sessions][fade]
   float* pin_emit = nullptr;       // pinned [max_sessions][2*chunk + fade]
+  // live-stream ingest (mc_pool_set_resampler / mc_pool_push_pcm): one polyphase plan per client rate, and the clients'
+  // raw chunks staged in pinned memory, read in place by pool_ingest_kernel
+  struct Resampler { int sr = 0, up = 1, down = 1, n_taps = 0; long long pre_remove = 0; float* taps = nullptr; };
+  std::vector<Resampler> resamplers;
+  unsigned char* pin_pcm = nullptr;
+  size_t pin_pcm_bytes = 0;
+  int pcm_max_in = 0, pcm_max_channels = 0;   // mc_pool_reserve_pcm's bounds (0: the staging grows when a call needs it)
+  PoolIngestItem* pin_items = nullptr;         // pinned [max_sessions]
 };
 
 namespace {
@@ -1674,6 +1682,90 @@ void ragged_decode_cut(const mc_pool* p, int n, int F_max, int hop, int keep, in
   *rows = ragged_cut((need + hop - 1) / hop + margin, F_max);
   *dec_keep = *rows >= F_max ? F_max * hop : (*rows - margin) * hop;
 }
+
+int pool_hop(const mc_pool* p) {
+  int hop = 1;
+  for (int i = 0; i < p->h->spec.n_convs; ++i) hop *= p->h->spec.conv_strides[i];
+  return hop;
+}
+
+// What mc_pool_push_audio and mc_pool_push_pcm share once the checks have passed and the new chunks are staged on the
+// host: `stage(stream)` enqueues what fills dev_chunk ([n*C][cap], len samples per row); the context roll, the encode
+// and the codes' way back follow in the same graph.  kind: the first element of the graph key.
+template <typename Stage>
+int pool_encode_uniform(mc_pool* p, const int32_t* slots, int n, int old_len, int len, int keep_frames, int64_t* codes_out,
+                        int32_t* frames_out, mc_stream_t stream_, int kind, Stage stage) {
+  mc_handle* h = p->h;
+  MC_CUDA(h, cudaEventRecord(p->order_ev, (cudaStream_t)stream_));
+  MC_CUDA(h, cudaStreamWaitEvent(p->own, p->order_ev, 0));
+  cudaStream_t stream = p->own;
+  const int hop = pool_hop(p);
+  const int C = p->C, cap = p->cap_samples, rows = n * C;
+  const int new_len = std::min(old_len + len, std::max(len, p->ctx_samples));
+  const int keep_old = new_len - len;
+  const int F = (new_len + hop - 1) / hop;
+  const int keep = (keep_frames <= 0 || keep_frames > F) ? F : keep_frames;
+  for (int j = 0; j < n; ++j) { p->pin_table[2 * j] = slots[j]; p->pin_table[2 * j + 1] = p->acur[slots[j]]; }
+  auto body = [&]() -> int {
+    MC_CUDA(h, cudaMemcpyAsync(p->dev_table, p->pin_table, (size_t)n * 8, cudaMemcpyHostToDevice, stream));
+    MC_TRY(stage(stream));
+    pool_roll_kernel<float><<<dim3((new_len + 255) / 256, rows), 256, 0, stream>>>(p->dev_table, C, cap, old_len, keep_old, len, p->audio[0],
+                                                                                  p->audio[1], p->dev_chunk, p->batch_audio, cap);
+    MC_LAUNCH_CHECK(h, "pool_roll_kernel");
+    MC_TRY(encode_impl(h, p->batch_audio, cap, rows, new_len, keep, p->dev_codes_out, nullptr, nullptr, stream));
+    MC_CUDA(h, cudaMemcpyAsync(p->pin_codes_out, p->dev_codes_out, (size_t)rows * keep * 8, cudaMemcpyDeviceToHost, stream));
+    return MC_OK;
+  };
+  MC_TRY(run_or_replay(p, std::make_tuple(kind, old_len, len, keep, n, 0), stream, body));
+  MC_CUDA(h, cudaStreamSynchronize(stream));
+  memcpy(codes_out, p->pin_codes_out, (size_t)rows * keep * 8);
+  if (frames_out) *frames_out = keep;
+  for (int j = 0; j < n; ++j) { p->acur[slots[j]] ^= 1; p->audio_len[slots[j]] = new_len; }
+  return MC_OK;
+}
+
+// The ragged counterpart (mc_pool_push_audio_ragged / mc_pool_push_pcm_ragged) for contexts of different length.
+template <typename Stage>
+int pool_encode_ragged(mc_pool* p, const int32_t* slots, int n, int len, int keep_frames, int64_t* codes_out, mc_stream_t stream_,
+                       int kind, Stage stage) {
+  mc_handle* h = p->h;
+  MC_CUDA(h, cudaEventRecord(p->order_ev, (cudaStream_t)stream_));
+  MC_CUDA(h, cudaStreamWaitEvent(p->own, p->order_ev, 0));
+  cudaStream_t stream = p->own;
+  const int hop = pool_hop(p);
+  const int C = p->C, cap = p->cap_samples, rows = n * C, keep = keep_frames;
+  const int T_max = pool_fill_ragged_table(p, slots, n, len, p->ctx_samples, p->audio_len, p->acur);
+  const int F_max = (T_max + hop - 1) / hop;
+  int F_min = F_max;
+  for (int j = 0; j < n; ++j) F_min = std::min(F_min, (p->pin_table[4 * j + 3] + hop - 1) / hop);
+  const int cut = ragged_cut(F_max - F_min + keep, F_max);
+  const RaggedKeep rg{p->dev_table, C, keep};
+  auto body = [&]() -> int {
+    MC_CUDA(h, cudaMemcpyAsync(p->dev_table, p->pin_table, (size_t)n * 16, cudaMemcpyHostToDevice, stream));
+    MC_TRY(stage(stream));
+    pool_roll_ragged_kernel<float><<<dim3((T_max + 255) / 256, rows), 256, 0, stream>>>(p->dev_table, C, cap, len, p->audio[0], p->audio[1],
+                                                                                       p->dev_chunk, p->batch_audio, cap, T_max);
+    MC_LAUNCH_CHECK(h, "pool_roll_ragged_kernel");
+    MC_TRY(encode_impl(h, p->batch_audio, cap, rows, T_max, cut, p->dev_codes_out, nullptr, nullptr, stream, &rg));
+    MC_CUDA(h, cudaMemcpyAsync(p->pin_codes_out, p->dev_codes_out, (size_t)rows * keep * 8, cudaMemcpyDeviceToHost, stream));
+    return MC_OK;
+  };
+  MC_TRY(run_or_replay(p, std::make_tuple(kind, T_max, len, cut, n, keep), stream, body));
+  MC_CUDA(h, cudaStreamSynchronize(stream));
+  memcpy(codes_out, p->pin_codes_out, (size_t)rows * keep * 8);
+  for (int j = 0; j < n; ++j) { p->acur[slots[j]] ^= 1; p->audio_len[slots[j]] = p->pin_table[4 * j + 3]; }
+  return MC_OK;
+}
+
+// mc_pool_push_audio's staging: the chunks go through pinned memory and one 2-D copy.
+void pool_stage_chunks_host(mc_pool* p, const float* chunks, int rows, int len) {
+  for (int r = 0; r < rows; ++r) memcpy(p->pin_chunk + (size_t)r * p->cap_samples, chunks + (size_t)r * len, (size_t)len * 4);
+}
+int pool_stage_chunks_device(mc_pool* p, int rows, int len, cudaStream_t stream) {
+  const size_t pitch = (size_t)p->cap_samples * 4;
+  MC_CUDA(p->h, cudaMemcpy2DAsync(p->dev_chunk, pitch, p->pin_chunk, pitch, (size_t)len * 4, rows, cudaMemcpyHostToDevice, stream));
+  return MC_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -1688,6 +1780,9 @@ int mc_pool_destroy(mc_pool* p) {
     if (d) cudaFree(d);
   for (void* q : {(void*)p->pin_chunk, (void*)p->pin_codes_in, (void*)p->pin_table, (void*)p->pin_codes_out, (void*)p->pin_wav_out})
     if (q) cudaFreeHost(q);
+  for (auto& r : p->resamplers) cudaFree(r.taps);
+  if (p->pin_pcm) cudaFreeHost(p->pin_pcm);
+  if (p->pin_items) cudaFreeHost(p->pin_items);
   if (p->order_ev) cudaEventDestroy(p->order_ev);
   if (p->own) cudaStreamDestroy(p->own);
   delete p;
@@ -1761,34 +1856,10 @@ int mc_pool_push_audio(mc_pool* p, const int32_t* slots, int32_t n, const float*
   MC_TRY(pool_check_slots(p, slots, n, p->audio_len, &old_len, "mc_pool_push_audio"));
   if (!chunks || !codes_out || len < 1) return h->fail(MC_ERR_ARG, "mc_pool_push_audio: bad arguments");
   if (len > p->cap_samples) return h->fail(MC_ERR_ARG, "mc_pool_push_audio: chunk of %d samples exceeds the capacity %d", len, p->cap_samples);
-  MC_CUDA(h, cudaEventRecord(p->order_ev, (cudaStream_t)stream_));
-  MC_CUDA(h, cudaStreamWaitEvent(p->own, p->order_ev, 0));
-  cudaStream_t stream = p->own;
-  int hop = 1;
-  for (int i = 0; i < h->spec.n_convs; ++i) hop *= h->spec.conv_strides[i];
-  const int C = p->C, cap = p->cap_samples, rows = n * C;
-  const int new_len = std::min(old_len + len, std::max(len, p->ctx_samples));
-  const int keep_old = new_len - len;
-  const int F = (new_len + hop - 1) / hop;
-  const int keep = (keep_frames <= 0 || keep_frames > F) ? F : keep_frames;
-  for (int r = 0; r < rows; ++r) memcpy(p->pin_chunk + (size_t)r * cap, chunks + (size_t)r * len, (size_t)len * 4);
-  for (int j = 0; j < n; ++j) { p->pin_table[2 * j] = slots[j]; p->pin_table[2 * j + 1] = p->acur[slots[j]]; }
-  auto body = [&]() -> int {
-    MC_CUDA(h, cudaMemcpyAsync(p->dev_table, p->pin_table, (size_t)n * 8, cudaMemcpyHostToDevice, stream));
-    MC_CUDA(h, cudaMemcpy2DAsync(p->dev_chunk, (size_t)cap * 4, p->pin_chunk, (size_t)cap * 4, (size_t)len * 4, rows, cudaMemcpyHostToDevice, stream));
-    pool_roll_kernel<float><<<dim3((new_len + 255) / 256, rows), 256, 0, stream>>>(p->dev_table, C, cap, old_len, keep_old, len, p->audio[0],
-                                                                                  p->audio[1], p->dev_chunk, p->batch_audio, cap);
-    MC_LAUNCH_CHECK(h, "pool_roll_kernel");
-    MC_TRY(encode_impl(h, p->batch_audio, cap, rows, new_len, keep, p->dev_codes_out, nullptr, nullptr, stream));
-    MC_CUDA(h, cudaMemcpyAsync(p->pin_codes_out, p->dev_codes_out, (size_t)rows * keep * 8, cudaMemcpyDeviceToHost, stream));
-    return MC_OK;
-  };
-  MC_TRY(run_or_replay(p, std::make_tuple(0, old_len, len, keep, n, 0), stream, body));
-  MC_CUDA(h, cudaStreamSynchronize(stream));
-  memcpy(codes_out, p->pin_codes_out, (size_t)rows * keep * 8);
-  if (frames_out) *frames_out = keep;
-  for (int j = 0; j < n; ++j) { p->acur[slots[j]] ^= 1; p->audio_len[slots[j]] = new_len; }
-  return MC_OK;
+  const int rows = n * p->C;
+  pool_stage_chunks_host(p, chunks, rows, len);
+  return pool_encode_uniform(p, slots, n, old_len, len, keep_frames, codes_out, frames_out, stream_, 0,
+                             [&](cudaStream_t st) { return pool_stage_chunks_device(p, rows, len, st); });
 }
 
 /* codes: HOST int64 [n][C][len]; wav_out: HOST fp32 [n][C][keep] (keep = keep_samples, or the whole window when 0). */
@@ -1943,38 +2014,15 @@ int mc_pool_push_audio_ragged(mc_pool* p, const int32_t* slots, int32_t n, const
   if (!chunks || !codes_out || len < 1) return h->fail(MC_ERR_ARG, "mc_pool_push_audio_ragged: bad arguments");
   if (len > p->cap_samples)
     return h->fail(MC_ERR_ARG, "mc_pool_push_audio_ragged: chunk of %d samples exceeds the capacity %d", len, p->cap_samples);
-  int hop = 1;
-  for (int i = 0; i < h->spec.n_convs; ++i) hop *= h->spec.conv_strides[i];
+  const int hop = pool_hop(p);
   if (keep_frames < 1 || keep_frames > (len + hop - 1) / hop)
     return h->fail(MC_ERR_ARG, "mc_pool_push_audio_ragged: keep_frames %d outside 1..%d", keep_frames, (len + hop - 1) / hop);
   if (common >= 0) return mc_pool_push_audio(p, slots, n, chunks, len, keep_frames, codes_out, nullptr, stream_);
   MC_TRY(pool_ragged_causal(p, "mc_pool_push_audio_ragged"));
-  MC_CUDA(h, cudaEventRecord(p->order_ev, (cudaStream_t)stream_));
-  MC_CUDA(h, cudaStreamWaitEvent(p->own, p->order_ev, 0));
-  cudaStream_t stream = p->own;
-  const int C = p->C, cap = p->cap_samples, rows = n * C, keep = keep_frames;
-  const int T_max = pool_fill_ragged_table(p, slots, n, len, p->ctx_samples, p->audio_len, p->acur);
-  const int F_max = (T_max + hop - 1) / hop;
-  int F_min = F_max;
-  for (int j = 0; j < n; ++j) F_min = std::min(F_min, (p->pin_table[4 * j + 3] + hop - 1) / hop);
-  const int cut = ragged_cut(F_max - F_min + keep, F_max);
-  for (int r = 0; r < rows; ++r) memcpy(p->pin_chunk + (size_t)r * cap, chunks + (size_t)r * len, (size_t)len * 4);
-  const RaggedKeep rg{p->dev_table, C, keep};
-  auto body = [&]() -> int {
-    MC_CUDA(h, cudaMemcpyAsync(p->dev_table, p->pin_table, (size_t)n * 16, cudaMemcpyHostToDevice, stream));
-    MC_CUDA(h, cudaMemcpy2DAsync(p->dev_chunk, (size_t)cap * 4, p->pin_chunk, (size_t)cap * 4, (size_t)len * 4, rows, cudaMemcpyHostToDevice, stream));
-    pool_roll_ragged_kernel<float><<<dim3((T_max + 255) / 256, rows), 256, 0, stream>>>(p->dev_table, C, cap, len, p->audio[0], p->audio[1],
-                                                                                       p->dev_chunk, p->batch_audio, cap, T_max);
-    MC_LAUNCH_CHECK(h, "pool_roll_ragged_kernel");
-    MC_TRY(encode_impl(h, p->batch_audio, cap, rows, T_max, cut, p->dev_codes_out, nullptr, nullptr, stream, &rg));
-    MC_CUDA(h, cudaMemcpyAsync(p->pin_codes_out, p->dev_codes_out, (size_t)rows * keep * 8, cudaMemcpyDeviceToHost, stream));
-    return MC_OK;
-  };
-  MC_TRY(run_or_replay(p, std::make_tuple(4, T_max, len, cut, n, keep), stream, body));
-  MC_CUDA(h, cudaStreamSynchronize(stream));
-  memcpy(codes_out, p->pin_codes_out, (size_t)rows * keep * 8);
-  for (int j = 0; j < n; ++j) { p->acur[slots[j]] ^= 1; p->audio_len[slots[j]] = p->pin_table[4 * j + 3]; }
-  return MC_OK;
+  const int rows = n * p->C;
+  pool_stage_chunks_host(p, chunks, rows, len);
+  return pool_encode_ragged(p, slots, n, len, keep_frames, codes_out, stream_, 4,
+                            [&](cudaStream_t st) { return pool_stage_chunks_device(p, rows, len, st); });
 }
 
 int mc_pool_push_codes_ragged(mc_pool* p, const int32_t* slots, int32_t n, const int64_t* codes, int32_t len, int32_t keep_samples,
@@ -2109,6 +2157,200 @@ int mc_pool_graph_count(mc_pool* p, int32_t* keys, int32_t* captured) {
   if (keys) *keys = (int32_t)p->graphs.size();
   if (captured) *captured = c;
   return MC_OK;
+}
+
+int mc_pool_read_audio(mc_pool* p, int32_t slot, float* out_host, int32_t n) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  if (slot < 0 || slot >= p->max_sessions || !out_host || n < 1 || n > p->audio_len[slot])
+    return h->fail(MC_ERR_ARG, "mc_pool_read_audio: need a slot < %d and 1 <= n <= its %d context samples", p->max_sessions,
+                   (slot >= 0 && slot < p->max_sessions) ? p->audio_len[slot] : 0);
+  const size_t cap = (size_t)p->cap_samples;
+  const float* src = p->audio[p->acur[slot]] + (size_t)slot * p->C * cap + (p->audio_len[slot] - n);
+  MC_CUDA(h, cudaMemcpy2DAsync(out_host, (size_t)n * 4, src, cap * 4, (size_t)n * 4, p->C, cudaMemcpyDeviceToHost, p->own));
+  MC_CUDA(h, cudaStreamSynchronize(p->own));
+  return MC_OK;
+}
+
+}  // extern "C"
+
+// ---- live-stream ingest: pooled sessions whose clients send s16 / f32 PCM at their own rate, [C_in][n] per chunk
+// (what AudioTokenizer._prep_audio_for_tokenization does on the host: int16 / 32768, the mean over channels for a mono
+// codec, the polyphase resampler), converted and resampled by pool_ingest_kernel inside the push's graph.
+namespace {
+size_t align16(size_t b) { return (b + 15) & ~(size_t)15; }
+size_t pcm_item_bytes(const mc_pcm_chunk& it) { return align16((size_t)it.channels_in * it.n_in * (it.format == PCM_S16 ? 2 : 4)); }
+
+// (Re)allocate the pinned payload staging.  The pcm graphs bake its address in, so they go; every other graph stays.
+int pool_pcm_alloc(mc_pool* p, size_t bytes, const char* what) {
+  mc_handle* h = p->h;
+  MC_CUDA(h, cudaStreamSynchronize(p->own));
+  for (auto it = p->graphs.begin(); it != p->graphs.end();) {
+    if (std::get<0>(it->first) >= 7) {
+      if (it->second.exec) cudaGraphExecDestroy(it->second.exec);
+      it = p->graphs.erase(it);
+    } else {
+      ++it;
+    }
+  }
+  if (p->pin_pcm) cudaFreeHost(p->pin_pcm);
+  p->pin_pcm = nullptr;
+  p->pin_pcm_bytes = 0;
+  cudaError_t e = cudaSuccess;
+  if (!p->pin_items) e = cudaMallocHost(&p->pin_items, (size_t)p->max_sessions * sizeof(PoolIngestItem));
+  if (e == cudaSuccess) e = cudaMallocHost(&p->pin_pcm, bytes);
+  if (e != cudaSuccess) { p->pin_pcm = nullptr; return h->fail(MC_ERR_NOMEM, "%s: %s", what, cudaGetErrorString(e)); }
+  p->pin_pcm_bytes = bytes;
+  return MC_OK;
+}
+
+const mc_pool::Resampler* pool_find_resampler(const mc_pool* p, int sr) {
+  for (const auto& r : p->resamplers)
+    if (r.sr == sr) return &r;
+  return nullptr;
+}
+
+// Every check of a pcm push's items, before any work or state change.
+int pool_check_pcm(mc_pool* p, int n, const mc_pcm_chunk* items, const void* payload, int len, const char* what) {
+  mc_handle* h = p->h;
+  if (!items || !payload || len < 1) return h->fail(MC_ERR_ARG, "%s: bad arguments", what);
+  if (len > p->cap_samples) return h->fail(MC_ERR_ARG, "%s: chunk of %d samples exceeds the capacity %d", what, len, p->cap_samples);
+  for (int j = 0; j < n; ++j) {
+    const mc_pcm_chunk& it = items[j];
+    if (it.format != PCM_S16 && it.format != PCM_F32)
+      return h->fail(MC_ERR_ARG, "%s: item %d: format %d (only MC_PCM_S16 and MC_PCM_F32)", what, j, it.format);
+    if (p->C > 1 && it.channels_in != p->C)
+      return h->fail(MC_ERR_ARG, "%s: item %d: %d channels for a %d-channel pool", what, j, it.channels_in, p->C);
+    if (p->C == 1 && (it.channels_in < 1 || it.channels_in > MC_POOL_MAX_MIX_CHANNELS))
+      return h->fail(MC_ERR_ARG, "%s: item %d: %d channels (a mono pool mixes 1..%d)", what, j, it.channels_in, MC_POOL_MAX_MIX_CHANNELS);
+    if (it.n_in < 1 || it.offset_bytes < 0 || (it.channels_in > 1 && it.ld < it.n_in))
+      return h->fail(MC_ERR_ARG, "%s: item %d: bad layout (n_in %d, ld %lld, offset %lld)", what, j, it.n_in, (long long)it.ld,
+                     (long long)it.offset_bytes);
+    if (p->pcm_max_in > 0 && (it.n_in > p->pcm_max_in || it.channels_in > p->pcm_max_channels))
+      return h->fail(MC_ERR_ARG, "%s: item %d: %d x %d samples exceed the staging reserved for %d x %d", what, j, it.channels_in, it.n_in,
+                     p->pcm_max_channels, p->pcm_max_in);
+    long long n_out = it.n_in;
+    if (it.sample_rate != h->spec.sample_rate) {
+      const mc_pool::Resampler* r = pool_find_resampler(p, it.sample_rate);
+      if (!r) return h->fail(MC_ERR_ARG, "%s: item %d: no resampler registered for %d Hz", what, j, it.sample_rate);
+      n_out = ((long long)it.n_in * r->up + r->down - 1) / r->down;
+    }
+    if (n_out != len)
+      return h->fail(MC_ERR_ARG, "%s: item %d: %d samples at %d Hz resample to %lld, the call's length is %d", what, j, it.n_in,
+                     it.sample_rate, n_out, len);
+  }
+  return MC_OK;
+}
+
+// Copy the items' rows into the pinned staging and fill the kernel's table.  Unless mc_pool_reserve_pcm fixed the staging,
+// it grows when a call needs more, to room for every slot at the call's largest item, so sessions that join do not
+// reallocate it (and drop the pcm graphs) again.
+int pool_stage_pcm_host(mc_pool* p, int n, const mc_pcm_chunk* items, const void* payload, const char* what) {
+  size_t total = 0, largest = 0;
+  for (int j = 0; j < n; ++j) { total += pcm_item_bytes(items[j]); largest = std::max(largest, pcm_item_bytes(items[j])); }
+  if (total > p->pin_pcm_bytes || !p->pin_items)
+    MC_TRY(pool_pcm_alloc(p, std::max(largest * p->max_sessions, 2 * p->pin_pcm_bytes), what));
+  size_t off = 0;
+  for (int j = 0; j < n; ++j) {
+    const mc_pcm_chunk& it = items[j];
+    const size_t es = it.format == PCM_S16 ? 2 : 4, row = (size_t)it.n_in * es;
+    for (int c = 0; c < it.channels_in; ++c)
+      memcpy(p->pin_pcm + off + c * row, static_cast<const unsigned char*>(payload) + it.offset_bytes + (size_t)c * it.ld * es, row);
+    PoolIngestItem& d = p->pin_items[j];
+    const mc_pool::Resampler* r = it.sample_rate != p->h->spec.sample_rate ? pool_find_resampler(p, it.sample_rate) : nullptr;
+    d.taps = r ? r->taps : nullptr;
+    d.offset = (long long)off;
+    d.pre_remove = r ? r->pre_remove : 0;
+    d.format = it.format; d.channels = it.channels_in; d.n_in = it.n_in;
+    d.up = r ? r->up : 1; d.down = r ? r->down : 1; d.n_taps = r ? r->n_taps : 0;
+    off += pcm_item_bytes(it);
+  }
+  return MC_OK;
+}
+
+int pool_stage_pcm_device(mc_pool* p, int n, int len, cudaStream_t stream) {
+  pool_ingest_kernel<<<dim3((len + INGEST_TILE - 1) / INGEST_TILE, n * p->C), 256, 0, stream>>>(p->pin_items, p->pin_pcm, p->C, len,
+                                                                                                  p->dev_chunk, p->cap_samples);
+  MC_LAUNCH_CHECK(p->h, "pool_ingest_kernel");
+  return MC_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int mc_pool_set_resampler(mc_pool* p, int32_t sr_in, int32_t up, int32_t down, const float* taps, int32_t n_taps, int64_t pre_remove) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  const int sr = h->spec.sample_rate;
+  if (sr_in < 1 || sr_in == sr || up < 1 || down < 1 || (int64_t)sr_in * up != (int64_t)sr * down || !taps || n_taps < 1 || pre_remove < 0)
+    return h->fail(MC_ERR_ARG, "mc_pool_set_resampler: bad plan (%d Hz -> %d Hz, up %d, down %d, %d taps)", sr_in, sr, up, down, n_taps);
+  if (ingest_span(up, down, n_taps) > INGEST_SPAN)
+    return h->fail(MC_ERR_ARG, "mc_pool_set_resampler: %d Hz: a tile reads %lld input samples, more than %d", sr_in,
+                   ingest_span(up, down, n_taps), INGEST_SPAN);
+  if (!pool_find_resampler(p, sr_in) && (int)p->resamplers.size() >= MC_POOL_MAX_RESAMPLERS)
+    return h->fail(MC_ERR_ARG, "mc_pool_set_resampler: already %d input rates registered", MC_POOL_MAX_RESAMPLERS);
+  float* d = nullptr;
+  cudaError_t e = cudaMalloc(&d, (size_t)n_taps * 4);
+  if (e == cudaSuccess) e = cudaMemcpy(d, taps, (size_t)n_taps * 4, cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) {
+    if (d) cudaFree(d);
+    return h->fail(MC_ERR_NOMEM, "mc_pool_set_resampler: %s", cudaGetErrorString(e));
+  }
+  MC_CUDA(h, cudaStreamSynchronize(p->own));   // a replaced plan's taps may still be read by the last push
+  mc_pool::Resampler* r = const_cast<mc_pool::Resampler*>(pool_find_resampler(p, sr_in));
+  if (!r) { p->resamplers.emplace_back(); r = &p->resamplers.back(); }
+  if (r->taps) cudaFree(r->taps);
+  r->sr = sr_in; r->up = up; r->down = down; r->n_taps = n_taps; r->pre_remove = pre_remove; r->taps = d;
+  return MC_OK;
+}
+
+int mc_pool_reserve_pcm(mc_pool* p, int32_t max_in_samples, int32_t max_in_channels) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  const int ch_limit = p->C > 1 ? p->C : MC_POOL_MAX_MIX_CHANNELS;
+  if (max_in_samples < 1 || max_in_channels < 1 || max_in_channels > ch_limit)
+    return h->fail(MC_ERR_ARG, "mc_pool_reserve_pcm: need max_in_samples >= 1 and 1 <= max_in_channels <= %d", ch_limit);
+  const size_t bytes = (size_t)p->max_sessions * align16((size_t)max_in_samples * max_in_channels * 4);
+  if (bytes != p->pin_pcm_bytes || !p->pin_items) MC_TRY(pool_pcm_alloc(p, bytes, "mc_pool_reserve_pcm"));
+  p->pcm_max_in = max_in_samples;
+  p->pcm_max_channels = max_in_channels;
+  return MC_OK;
+}
+
+int mc_pool_push_pcm(mc_pool* p, const int32_t* slots, int32_t n, const mc_pcm_chunk* items, const void* payload, int32_t len,
+                     int32_t keep_frames, int64_t* codes_out, int32_t* frames_out, mc_stream_t stream_) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  int old_len = 0;
+  MC_TRY(pool_check_slots(p, slots, n, p->audio_len, &old_len, "mc_pool_push_pcm"));
+  if (!codes_out) return h->fail(MC_ERR_ARG, "mc_pool_push_pcm: bad arguments");
+  MC_TRY(pool_check_pcm(p, n, items, payload, len, "mc_pool_push_pcm"));
+  MC_TRY(pool_stage_pcm_host(p, n, items, payload, "mc_pool_push_pcm"));
+  return pool_encode_uniform(p, slots, n, old_len, len, keep_frames, codes_out, frames_out, stream_, 7,
+                             [&](cudaStream_t st) { return pool_stage_pcm_device(p, n, len, st); });
+}
+
+int mc_pool_push_pcm_ragged(mc_pool* p, const int32_t* slots, int32_t n, const mc_pcm_chunk* items, const void* payload, int32_t len,
+                            int32_t keep_frames, int64_t* codes_out, mc_stream_t stream_) {
+  if (!p) return MC_ERR_ARG;
+  mc_handle* h = p->h;
+  MC_ENTER(h);
+  int common = 0;
+  MC_TRY(pool_check_slots(p, slots, n, p->audio_len, &common, "mc_pool_push_pcm_ragged", false));
+  if (!codes_out) return h->fail(MC_ERR_ARG, "mc_pool_push_pcm_ragged: bad arguments");
+  MC_TRY(pool_check_pcm(p, n, items, payload, len, "mc_pool_push_pcm_ragged"));
+  const int hop = pool_hop(p);
+  if (keep_frames < 1 || keep_frames > (len + hop - 1) / hop)
+    return h->fail(MC_ERR_ARG, "mc_pool_push_pcm_ragged: keep_frames %d outside 1..%d", keep_frames, (len + hop - 1) / hop);
+  if (common >= 0) return mc_pool_push_pcm(p, slots, n, items, payload, len, keep_frames, codes_out, nullptr, stream_);
+  MC_TRY(pool_ragged_causal(p, "mc_pool_push_pcm_ragged"));
+  MC_TRY(pool_stage_pcm_host(p, n, items, payload, "mc_pool_push_pcm_ragged"));
+  return pool_encode_ragged(p, slots, n, len, keep_frames, codes_out, stream_, 8,
+                            [&](cudaStream_t st) { return pool_stage_pcm_device(p, n, len, st); });
 }
 
 }  // extern "C"

@@ -132,4 +132,72 @@ resample_poly_kernel(const float* __restrict__ x, long long in_ld, int C, long l
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Live-stream ingest of a session-pool push (mc_pool_push_pcm): every item of the batch is one client's raw chunk (s16 or
+// f32, planar [channels][n_in], at its own rate) and becomes the item's fp32 rows of the pool's chunk staging at the
+// codec's rate, which pool_roll_kernel / pool_roll_ragged_kernel then read as for mc_pool_push_audio.  Per item and
+// output channel the values are bit for bit those of pcm_to_f32_kernel (mixing to mono when a mono pool gets several
+// channels) followed by resample_poly_kernel on the same bytes: the same conversion and mean, and the same FMA order.
+// ---------------------------------------------------------------------------------------------
+constexpr int INGEST_TILE = 256;    // outputs per CTA
+constexpr int INGEST_SPAN = 8192;   // input samples a CTA holds in shared memory (the host checks each plan's span fits)
+
+struct PoolIngestItem {             // one per batch item, read in place from pinned host memory
+  const float* taps;                // device taps of the item's rate (resample_poly_kernel's h); NULL: the codec's rate
+  long long offset;                 // byte offset of the item's rows [channels][n_in] in the staged payload
+  long long pre_remove;
+  int format, channels, n_in, up, down, n_taps;
+};
+
+// Input samples a tile of INGEST_TILE outputs can read: (TILE - 1) * down / up + 1 bases, (n_taps - 1) / up older ones.
+__host__ __device__ inline long long ingest_span(int up, int down, int n_taps) {
+  return static_cast<long long>(INGEST_TILE - 1) * down / up + (n_taps - 1) / up + 2;
+}
+
+// grid (ceil(n_out / INGEST_TILE), n * C_out); out: [n * C_out][out_ld], row j * C_out + c.
+__global__ void __launch_bounds__(256)
+pool_ingest_kernel(const PoolIngestItem* __restrict__ items, const unsigned char* __restrict__ payload, int C_out, int n_out,
+                   float* __restrict__ out, int out_ld) {
+  __shared__ float xs[INGEST_SPAN];
+  const int jc = blockIdx.y, j = jc / C_out, c = jc - j * C_out;
+  const PoolIngestItem it = items[j];
+  const unsigned char* src = payload + it.offset;
+  const bool mix = C_out == 1 && it.channels > 1;            // a mono pool fed several channels: np.mean(axis=0) in fp32
+  const long long row = mix ? 0 : static_cast<long long>(c) * it.n_in;
+  auto sample = [&](long long t) -> float {
+    if (!mix) return pcm_sample(src, it.format, row + t, 0);
+    float acc = 0.0f;
+    for (int k = 0; k < it.channels; ++k) acc += pcm_sample(src, it.format, static_cast<long long>(k) * it.n_in + t, 0);
+    return acc / static_cast<float>(it.channels);
+  };
+  const long long i0 = static_cast<long long>(blockIdx.x) * INGEST_TILE;
+  const long long i1 = min(i0 + INGEST_TILE, static_cast<long long>(n_out));
+  float* o = out + static_cast<long long>(jc) * out_ld;
+  if (it.taps == nullptr) {                                    // the codec's rate: conversion only
+    for (long long i = i0 + threadIdx.x; i < i1; i += blockDim.x) o[i] = sample(i);
+    return;
+  }
+  const int up = it.up, down = it.down, n_taps = it.n_taps;
+  const long long n_in = it.n_in;
+  // the tile reads input samples [lo, hi]: base - j with base = (i + pre) * down / up and 0 <= j <= (n_taps - 1) / up
+  const long long lo = max(0LL, (i0 + it.pre_remove) * down / up - (n_taps - 1) / up);
+  const long long hi = min(n_in - 1, (i1 - 1 + it.pre_remove) * down / up);
+  for (long long t = lo + threadIdx.x; t <= hi; t += blockDim.x) xs[t - lo] = sample(t);
+  __syncthreads();
+  const float* __restrict__ h = it.taps;
+  for (long long i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+    // resample_poly_kernel's loop, reading the converted samples from shared memory
+    const long long t = (i + it.pre_remove) * down;
+    const int phase = static_cast<int>(t % up);
+    const long long base = t / up;
+    long long j0 = base >= n_in ? base - (n_in - 1) : 0;
+    long long j1 = (n_taps - 1 - phase) / up;
+    if (base < j1) j1 = base;
+    float acc = 0.0f;
+#pragma unroll 8   // the tap loads of 8 steps in flight; the FMAs stay in resample_poly_kernel's order
+    for (long long jj = j0; jj <= j1; ++jj) acc = fmaf(__ldg(h + phase + jj * up), xs[base - jj - lo], acc);
+    o[i] = acc;
+  }
+}
+
 }  // namespace mc

@@ -32,6 +32,8 @@ from typing import Dict, List, Optional, Tuple
 import numpy as np
 
 from . import _native as nat
+from . import audio_io as aio
+from .audio_tokenizer import prep_audio_for_tokenization
 from .audio_utils import create_crossfade_ramps
 from .codec_chars import UNICODE_OFFSET_LARGE, chars_to_codes, codes_to_chars
 
@@ -145,6 +147,69 @@ class SessionPool:
             nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_push_codes_emit_ragged")
         return out, had.astype(bool)
 
+    def set_resampler(self, sr_in: int, plan) -> None:
+        """Register the polyphase plan of one client rate for push_pcm (mc_pool_set_resampler): the ResamplePlan of
+        audio_io.resample_plan(sr_in, codec rate)."""
+        taps = np.ascontiguousarray(plan.taps, dtype=np.float32)
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_set_resampler(self._p, int(sr_in), plan.up, plan.down, taps.ctypes.data, taps.size,
+                                                     plan.pre_remove)
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_set_resampler")
+
+    def reserve_pcm(self, max_in_samples: int, max_in_channels: int) -> None:
+        """Fix push_pcm's pinned staging at max_in_channels x max_in_samples per session (mc_pool_reserve_pcm)."""
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_reserve_pcm(self._p, int(max_in_samples), int(max_in_channels))
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_reserve_pcm")
+
+    @staticmethod
+    def _pcm_items(pcm) -> Tuple[np.ndarray, np.ndarray]:
+        """[(sr, int16 / float32 [T] or [C_in, T])] -> (mc_pcm_chunk table, payload bytes)."""
+        items = np.zeros(len(pcm), dtype=nat.PCM_CHUNK_DTYPE)
+        parts, off = [], 0
+        for j, (sr, x) in enumerate(pcm):
+            x = np.ascontiguousarray(x)
+            if x.dtype not in (np.int16, np.float32) or x.ndim not in (1, 2):
+                raise ValueError(f"item {j}: push_pcm takes int16 / float32 [T] or [C_in, T], got {x.dtype} {x.shape}")
+            rows = x.reshape(-1, x.shape[-1])
+            items[j] = (aio.PCM_S16 if x.dtype == np.int16 else aio.PCM_F32, rows.shape[0], rows.shape[1], int(sr), off, rows.shape[1])
+            parts.append(rows.reshape(-1).view(np.uint8))
+            off += rows.nbytes
+        return items, np.concatenate(parts) if parts else np.zeros(1, np.uint8)
+
+    def push_pcm(self, slots, pcm, length: int, keep_frames: int) -> np.ndarray:
+        """push_audio on raw client chunks: pcm = [(sr, int16 / float32 [T] or [C_in, T])], each at the codec's rate or a
+        registered one and resampling to `length` samples; converted, mixed and resampled on the device -> int64 codes
+        [n, C, keep]."""
+        slots = np.ascontiguousarray(slots, dtype=np.int32)
+        items, payload = self._pcm_items(pcm)
+        out = np.empty((len(slots) * self.channels * self.cap_frames,), dtype=np.int64)
+        got = C.c_int32(0)
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_push_pcm(self._p, slots.ctypes.data, len(slots), items.ctypes.data, payload.ctypes.data, int(length),
+                                                keep_frames, out.ctypes.data, C.byref(got), self.gen._stream())
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_push_pcm")
+        return out[: len(slots) * self.channels * got.value].reshape(len(slots), self.channels, got.value)
+
+    def push_pcm_ragged(self, slots, pcm, length: int, keep_frames: int) -> np.ndarray:
+        """push_audio_ragged on raw client chunks (see push_pcm) -> int64 codes [n, C, keep_frames]."""
+        slots = np.ascontiguousarray(slots, dtype=np.int32)
+        items, payload = self._pcm_items(pcm)
+        out = np.empty((len(slots), self.channels, keep_frames), dtype=np.int64)
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_push_pcm_ragged(self._p, slots.ctypes.data, len(slots), items.ctypes.data, payload.ctypes.data,
+                                                       int(length), keep_frames, out.ctypes.data, self.gen._stream())
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_push_pcm_ragged")
+        return out
+
+    def read_audio(self, slot: int, n: int) -> np.ndarray:
+        """The last n samples of a slot's audio context, float32 [C, n] (mc_pool_read_audio)."""
+        out = np.empty((self.channels, n), dtype=np.float32)
+        with self.gen._serial():
+            rc = self.gen._lib.mc_pool_read_audio(self._p, int(slot), out.ctypes.data, int(n))
+            nat.check(self.gen._lib, self.gen._handle, rc, "mc_pool_read_audio")
+        return out
+
     def graph_count(self) -> Tuple[int, int]:
         """(distinct graph keys seen, graphs captured) over every push of this pool."""
         k, c = C.c_int32(), C.c_int32()
@@ -193,6 +258,7 @@ class SessionBatcher:
         self._next_id = 0
         self._lock = threading.RLock()
         self._emit: Optional[Tuple[int, int]] = None   # (chunk samples, fade samples) once arm_emit ran
+        self._rates: set = set()                       # client rates whose resampler the pool holds
 
     # ---- session lifetime
     def open_session(self) -> int:
@@ -217,35 +283,63 @@ class SessionBatcher:
             st.audio_len, st.detok_context, st.history = 0, "", []
 
     # ---- encode
-    def tokenize_audio(self, chunks: Dict[int, np.ndarray]) -> Dict[int, str]:
-        """{session: float32/int16 chunk [T] or [C,T] at the codec's rate} -> {session: code string}, each exactly what
-        that session's AudioTokenizer.tokenize_audio (audio_tokenizer.py:67-103) would return."""
+    def tokenize_audio(self, chunks: Dict[int, object]) -> Dict[int, str]:
+        """{session: chunk} -> {session: code string}, each exactly what that session's AudioTokenizer.tokenize_audio
+        (audio_tokenizer.py:67-103) would return for the same chunk.  A chunk is what AudioTokenizer takes: a float32/int16
+        array [T] or [C,T] at the codec's rate, or an (sr, array) tuple.  Tuples of int16 data, or of float32 data at another
+        rate, are converted, mixed and resampled on the device inside the push (SessionPool.push_pcm; the first chunk at a
+        new rate registers its resampler); every other chunk is prepared on the host as AudioTokenizer does.  When a group
+        holds such a tuple, all its chunks go through push_pcm, so a tick stays one engine call per group."""
         C_ = self.num_channels
         with self._lock:
             groups: Dict[Tuple[int, int], List[int]] = {}
-            prepped = {}
+            prepped, raw, rates = {}, {}, set()
             for sid, chunk in chunks.items():                    # validate everything before any state changes
                 if sid not in self._sessions:
                     raise KeyError(f"unknown session {sid}")
-                x = np.asarray(chunk)
-                if x.dtype == np.int16:
-                    x = x.astype("float32") / 32768.0
-                if C_ == 1 and x.ndim > 1:
-                    x = np.mean(x, axis=0)
-                x = np.ascontiguousarray(x, dtype=np.float32).reshape(C_, -1)
-                if not 0 < x.shape[1] <= self.pool.cap_samples:
-                    raise ValueError(f"session {sid}: chunks must hold 1..{self.pool.cap_samples} samples")
-                prepped[sid] = x
+                ingest = self._device_ingest(chunk)
+                if ingest is not None:
+                    sr, x = raw[sid] = ingest
+                    if sr == self.sampling_rate:
+                        n_new = x.shape[-1]
+                    else:
+                        n_new = aio.resample_plan(sr, self.sampling_rate).n_out(x.shape[-1])
+                        rates.add(sr)
+                else:
+                    if isinstance(chunk, tuple):
+                        x = prep_audio_for_tokenization((int(chunk[0]), np.asarray(chunk[1])), self.sampling_rate, C_)
+                    else:
+                        x = np.asarray(chunk)
+                        if x.dtype == np.int16:
+                            x = x.astype("float32") / 32768.0
+                        if C_ == 1 and x.ndim > 1:
+                            x = np.mean(x, axis=0)
+                    x = np.ascontiguousarray(x, dtype=np.float32).reshape(C_, -1)
+                    n_new = x.shape[1]
+                    prepped[sid] = x
+                if not 0 < n_new <= self.pool.cap_samples:
+                    raise ValueError(f"session {sid}: chunks must hold 1..{self.pool.cap_samples} samples at {self.sampling_rate} Hz")
                 # ragged: one call per chunk length; the [-0:] case keeps every frame of each window, so it stays grouped
-                ragged = self.ragged and self._n_chars(x.shape[1]) > 0
-                groups.setdefault((-1 if ragged else self._sessions[sid].audio_len, x.shape[1]), []).append(sid)
+                ragged = self.ragged and self._n_chars(n_new) > 0
+                groups.setdefault((-1 if ragged else self._sessions[sid].audio_len, n_new), []).append(sid)
+            if len(self._rates | rates) > nat.MC_POOL_MAX_RESAMPLERS:
+                raise ValueError(f"a session pool converts at most {nat.MC_POOL_MAX_RESAMPLERS} client rates on the device, "
+                                 f"this tick would need {sorted(self._rates | rates)}")
+            for sr in sorted(rates - self._rates):
+                self.pool.set_resampler(sr, aio.resample_plan(sr, self.sampling_rate))
+                self._rates.add(sr)
             out: Dict[int, str] = {}
             for (ctx_len, n_new), sids in groups.items():
                 n_chars = self._n_chars(n_new)
                 frames_needed = -(-n_chars // C_) if n_chars > 0 else 0                  # 0 -> all frames ([-0:])
                 slots = [self._sessions[s].slot for s in sids]
-                push = self.pool.push_audio_ragged if ctx_len < 0 else self.pool.push_audio
-                codes = push(slots, np.stack([prepped[s] for s in sids]), frames_needed)   # [n,C,k]
+                if any(s in raw for s in sids):
+                    push = self.pool.push_pcm_ragged if ctx_len < 0 else self.pool.push_pcm
+                    pcm = [raw[s] if s in raw else (self.sampling_rate, prepped[s]) for s in sids]
+                    codes = push(slots, pcm, n_new, frames_needed)                       # [n,C,k]
+                else:
+                    push = self.pool.push_audio_ragged if ctx_len < 0 else self.pool.push_audio
+                    codes = push(slots, np.stack([prepped[s] for s in sids]), frames_needed)   # [n,C,k]
                 for j, sid in enumerate(sids):
                     st = self._sessions[sid]
                     st.audio_len = min(st.audio_len + n_new, max(n_new, self.context_samples))
@@ -253,6 +347,21 @@ class SessionBatcher:
                     text = codes_to_chars(frame_major, self.codebook_size, unicode_offset=self.unicode_offset)
                     out[sid] = text[-n_chars:]
             return out
+
+    def _device_ingest(self, chunk) -> Optional[Tuple[int, np.ndarray]]:
+        """(sr, array) when the chunk is converted on the device: an (sr, int16 / float32 array) tuple that needs more than a
+        cast (int16 data, or another rate) and has a shape the pool takes ([T] or [1..8, T] on a mono pool, [C, T] else);
+        None for everything the host prepares."""
+        if not isinstance(chunk, tuple) or len(chunk) != 2:
+            return None
+        sr, x = int(chunk[0]), np.asarray(chunk[1])
+        if x.dtype not in (np.int16, np.float32) or sr <= 0 or (x.dtype == np.float32 and sr == self.sampling_rate):
+            return None
+        if self.num_channels == 1:
+            fits = x.ndim == 1 or (x.ndim == 2 and 1 <= x.shape[0] <= nat.MC_POOL_MAX_MIX_CHANNELS)
+        else:
+            fits = x.ndim == 2 and x.shape[0] == self.num_channels
+        return (sr, x) if fits else None
 
     def _n_chars(self, n_new: int) -> int:
         return int(n_new / self.sampling_rate * self.framerate * self.num_channels)
@@ -389,7 +498,8 @@ class ThreadedSessionBatcher(SessionBatcher):
             self._cv.notify()
         return fut.result(timeout=timeout)
 
-    def tokenize_audio_one(self, sid: int, chunk: np.ndarray, timeout: Optional[float] = 30.0) -> str:
+    def tokenize_audio_one(self, sid: int, chunk, timeout: Optional[float] = 30.0) -> str:
+        """chunk: an array at the codec's rate or an (sr, array) tuple, as SessionBatcher.tokenize_audio takes it."""
         return self._submit(("encode",), sid, chunk, timeout)
 
     def detokenize_audio_one(self, sid: int, code_str: str, preroll_samples: int = 0, timeout: Optional[float] = 30.0):
